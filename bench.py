@@ -2,6 +2,7 @@
 """bench.py - seconds per Vicuna-7B block pruned (BASELINE.json metric), one JSON line on stdout.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--method wanda_nm|wanda_unstructured|sparsegpt|dsnot]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...     # the unmodified reference on the host cores (oracle/ref_arm.py; port fallback)
 
@@ -466,7 +467,25 @@ GRAPH_METHODS = ("wanda_nm", "wanda_unstructured", "dsnot", "dsnot_elided", "wan
                                                                 # conditional damping reads a status word)
 
 
-def time_method(ctx, method, inputs, steps, warmup, sample_clocks, dist, use_graph=True):
+DUMP_ROWS = 128     # rows per linear in --dump-outputs: the 7 weights + masks of a block in 35 MB
+DUMP_SEED = 200     # weight set of the last timed step of either pass when outputs are kept: same inputs in both passes
+
+
+def sample_outputs(torch, weights, masks):
+    """{file name: float32 array} of what a caller of one step receives: every pruned weight and, for the methods that
+    return them, the keep masks, each cut to the same DUMP_ROWS rows (a fixed seeded choice per linear)."""
+    import numpy as np
+    out = {}
+    for li, (name, R, _, _) in enumerate(LINEARS):
+        W = weights[name]
+        rows = torch.from_numpy(np.sort(np.random.default_rng(li).choice(R, DUMP_ROWS, replace=False))).to(W.device)
+        out[f"{name}.weight"] = W.index_select(0, rows).float().cpu().numpy()
+        if masks:
+            out[f"{name}.mask"] = masks[name].index_select(0, rows).float().cpu().numpy()
+    return out
+
+
+def time_method(ctx, method, inputs, steps, warmup, sample_clocks, dist, use_graph=True, keep_outputs=False):
     """W untimed + K timed steps of one method, a fresh weight set per step.
 
     Pass A (eager launches): per-span CUDA events -> the kernel shares behind `roofline`.
@@ -474,6 +493,8 @@ def time_method(ctx, method, inputs, steps, warmup, sample_clocks, dist, use_gra
     graph (kernels + NCCL collectives) and replayed once inside the timed region: neither the Python launch overhead
     (~100 small launches per 3 ms step) nor the host's graph-launch latency between steps (0.15-0.2 ms, measured)
     sits between the steps.  The headline is the faster of the two passes (both time exactly K steps on the device, max over ranks).
+    keep_outputs: the last timed step of each pass prunes a fresh weight set of seed DUMP_SEED, and out["outputs"] holds
+    sample_outputs() of that step in the pass behind the headline (out["outputs_pass"]), taken after both passes.
     Returns dict(ms_per_step, launches, kernels, ...)."""
     torch = ctx.torch
     nsets = min(steps + warmup, 24)
@@ -511,13 +532,18 @@ def time_method(ctx, method, inputs, steps, warmup, sample_clocks, dist, use_gra
     # ---- pass A: eager, with per-span events on the launching stream
     sampler = ClockSampler(ctx.dev.index)
     ctx.events = None
+    last = {}                                # pass -> (weights, masks) of its last timed step, with keep_outputs
+    wlast = make_block(torch, ctx.dev, seed=DUMP_SEED) if keep_outputs else None
 
     def eager_step(i):
         if i == warmup:                      # the timed region starts here
             ctx.events, ctx.launches = [], 0
             if sample_clocks:
                 sampler.start()
-        run_step(ctx, method, wsets[i % nsets], inputs)
+        w = wlast if wlast is not None and i == warmup + steps - 1 else wsets[i % nsets]
+        masks = run_step(ctx, method, w, inputs)
+        if w is wlast:
+            last["eager"] = (w, masks)
     eager_ms = timed_loop(eager_step)
     clocks = sampler.stop() if sample_clocks else None
     kern = {}
@@ -538,18 +564,23 @@ def time_method(ctx, method, inputs, steps, warmup, sample_clocks, dist, use_gra
             torch.cuda.empty_cache()
             nsets = min(steps, 24)
             wsets = [make_block(torch, ctx.dev, seed=100 + s) for s in range(nsets)]
+            wlast = make_block(torch, ctx.dev, seed=DUMP_SEED) if keep_outputs else None
             barrier()
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
                 for i in range(steps):
-                    run_step(ctx, method, wsets[i % nsets], inputs)
+                    w = wlast if wlast is not None and i == steps - 1 else wsets[i % nsets]
+                    masks = run_step(ctx, method, w, inputs)
             barrier()
             # warm-up: whole replays (K >= 1 steps each, at least W steps in all; the first one also uploads the graph to
             # the device), then the weights the warm replays pruned are restored (the selection kernels are data dependent)
             for _ in range(max(1, -(-warmup // steps))):
                 g.replay()
-            for si, w in enumerate(wsets):
-                for name, t in make_block(torch, ctx.dev, seed=100 + si).items():
+            restore = [(100 + si, w) for si, w in enumerate(wsets)]
+            if wlast is not None:
+                restore.append((DUMP_SEED, wlast))
+            for seed, w in restore:
+                for name, t in make_block(torch, ctx.dev, seed=seed).items():
                     w[name].copy_(t)
             barrier()
             sampler = ClockSampler(ctx.dev.index)
@@ -566,6 +597,9 @@ def time_method(ctx, method, inputs, steps, warmup, sample_clocks, dist, use_gra
             graph_ms = float(ms.item()) / steps
             out["graph_ms_per_step"] = graph_ms
             gclocks = sampler.stop() if sample_clocks else None
+            if keep_outputs:
+                last["graph"] = (wlast, masks)
+            del masks, wlast
             # both passes time exactly K steps on the device, max over ranks; the headline is the faster way of launching
             # the same work (at 8 GPUs the replay of a graph that holds NCCL collectives measured SLOWER than eager launches)
             if graph_ms <= out["ms_per_step"]:
@@ -578,7 +612,10 @@ def time_method(ctx, method, inputs, steps, warmup, sample_clocks, dist, use_gra
         except Exception as e:  # noqa: BLE001  (capture unsupported somewhere: the eager number stands)
             out["cuda_graph_error"] = f"{type(e).__name__}: {e}"[:200]
             torch.cuda.synchronize()
-    del wsets
+    if keep_outputs:
+        out["outputs_pass"] = "graph" if out["cuda_graph"] else "eager"
+        out["outputs"] = sample_outputs(torch, *last[out["outputs_pass"]])
+    del wsets, last
     torch.cuda.empty_cache()
     return out
 
@@ -697,7 +734,13 @@ def run_gpu(args):
         print(json.dumps({"one_step": args.method}), flush=True)
         return
 
-    main = time_method(ctx, args.method, inputs, args.steps, args.warmup, rank == 0, dist, not args.no_graph)
+    main = time_method(ctx, args.method, inputs, args.steps, args.warmup, rank == 0, dist, not args.no_graph,
+                       keep_outputs=args.dump_outputs is not None)
+    if args.dump_outputs is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in main.pop("outputs").items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     others = {}
     if args.all_methods:
         for m in METHODS:
@@ -754,6 +797,8 @@ def run_gpu(args):
             "config": {"workload": f"{WORKLOAD[args.method]} on one InstructBLIP-Vicuna-7B LLM block (7 linears, fp16 "
                                    f"weights, random init), {N_SEQ}x{SEQ_LEN} fp16 calibration tokens per linear",
                        "method": args.method, "calib_batch": args.calib_batch, "cuda_graph": main["cuda_graph"],
+                       "dump_outputs": {"dir": args.dump_outputs, "pass": main["outputs_pass"], "weight_seed": DUMP_SEED,
+                                        "rows_per_linear": DUMP_ROWS} if args.dump_outputs is not None else None,
                        "eager_ms_per_step": main["eager_ms_per_step"], "eager_step_ms": main["eager_step_ms"],
                        "graph_ms_per_step": main.get("graph_ms_per_step"), "weight_sets": main["weight_sets"],
                        "l2": "inputs larger than L2 (12.2 GB of activations per step, fresh weight set per step)",
@@ -1533,24 +1578,19 @@ def cpu_baseline(method):
 
 def run_reference(args):
     """`--impl reference`: the reference's own CPU implementation of the step on all host cores.  A step is the whole
-    block for the Wanda methods; the number of timed steps is capped so the run ends within a few minutes."""
+    block for the Wanda methods."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
     threads = os.cpu_count() or 1
     vals, sample, kind = [], "", "port"
-    t_start = time.perf_counter()
     warm = 0
     if args.warmup > 0:
         total, sample, kind = cpu_block_seconds(args.method, threads)       # one untimed pass: page cache, thread pool
         warm = 1
-    k = max(1, args.steps)
-    for i in range(k):
+    for _ in range(args.steps):
         total, sample, kind = cpu_block_seconds(args.method, threads)
         vals.append(total)
-        spent = time.perf_counter() - t_start
-        if spent + spent / (len(vals) + warm) > 170.0:                     # next step would pass ~3 minutes
-            break
     v = sum(vals) / len(vals)
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT,
@@ -1558,8 +1598,7 @@ def run_reference(args):
         "higher_is_better": False, "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": f"{WORKLOAD[args.method]} on one InstructBLIP-Vicuna-7B LLM block (7 linears, fp16 weights, "
                                f"random init), {N_SEQ}x{SEQ_LEN} fp16 calibration tokens per linear",
-                   "method": args.method, "steps_requested": args.steps,
-                   "steps_note": "timed steps capped so that the whole run stays within ~3 minutes"},
+                   "method": args.method},
         "cpu_baseline": {"value": v, "unit": UNIT, "cores": threads, "kind": kind, "sample": "each step: " + sample},
         "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0}), flush=True)
@@ -1580,7 +1619,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="time eager launches only (no CUDA-graph replay pass)")
     ap.add_argument("--no-other-methods", dest="all_methods", action="store_false",
                     help="skip the short measurement of the methods other than --method")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of --method returned (pruned weights, keep masks; the same "
+                         f"{DUMP_ROWS} seeded rows of every linear) as DIR/<linear>.<weight|mask>.npy, float32; one GPU only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "vlmc" or args.gpus != 1 or args.one_step):
+        ap.error("--dump-outputs needs --impl vlmc, --gpus 1 and timed steps")
     if args.warmup < 3 and args.impl == "vlmc":
         args.warmup = 3
     if args.impl == "reference":

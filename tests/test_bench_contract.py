@@ -46,6 +46,59 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_dump_outputs_sample(monkeypatch):
+    """--dump-outputs: float32 copies of the same seeded rows of every linear on every call, masks only when the method
+    returns them, at most 64 MB for the benched block; a run without timed steps or on several GPUs is refused up front."""
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    import torch
+    import bench
+    assert sum(2 * bench.DUMP_ROWS * C * 4 for _, _, C, _ in bench.LINEARS) <= 64 << 20
+    monkeypatch.setattr(bench, "LINEARS", [("a", 300, 40, "x"), ("b", 129, 24, "y")])
+    g = torch.Generator().manual_seed(0)
+    W = {n: torch.randn(R, C, generator=g).half() for n, R, C, _ in bench.LINEARS}
+    M = {n: torch.rand(R, C, generator=g) < 0.5 for n, R, C, _ in bench.LINEARS}
+    got = bench.sample_outputs(torch, W, M)
+    assert sorted(got) == ["a.mask", "a.weight", "b.mask", "b.weight"]
+    for n, R, C, _ in bench.LINEARS:
+        w, m = got[f"{n}.weight"], got[f"{n}.mask"]
+        assert w.dtype == m.dtype == np.float32 and w.shape == m.shape == (bench.DUMP_ROWS, C)
+        rows = [r for r in range(R) if any(np.array_equal(W[n][r].float().numpy(), x) for x in w)]
+        assert len(rows) == bench.DUMP_ROWS and np.array_equal(m, M[n][rows].float().numpy())
+    again = bench.sample_outputs(torch, W, None)
+    assert sorted(again) == ["a.weight", "b.weight"] and all(np.array_equal(again[k], got[k]) for k in again)
+    for bad in (["--steps", "0"], ["--gpus", "2", "--dump-outputs", "out"], ["--impl", "reference", "--dump-outputs", "out"]):
+        r = _run({}, *bad)
+        assert r.returncode == 2 and "error" in r.stderr, bad
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_timed_step(tmp_path):
+    """bench.py --dump-outputs end to end, Wanda 2:4: the graph replay and the eager pass each dump their last timed step;
+    both prune the same weight set, so the files are identical, and every dumped row is a 2:4 mask with the weight zero
+    wherever the mask drops it."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    dumps = {}
+    for graph in (True, False):
+        d = tmp_path / ("graph" if graph else "eager")
+        r = _run({}, "--steps", "2", "--warmup", "3", "--no-other-methods", "--no-cpu-baseline", "--no-full-model",
+                 "--dump-outputs", str(d), *([] if graph else ["--no-graph"]))
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads(r.stdout.strip().splitlines()[-1])
+        assert line["steps"] == 2 and line["config"]["dump_outputs"]["pass"] == ("graph" if graph else "eager")
+        assert sorted(p.name for p in d.iterdir()) == sorted(f"{n}.{k}.npy" for n, *_ in bench.LINEARS for k in ("weight", "mask"))
+        dumps[graph] = {p.name: np.load(p) for p in d.iterdir()}
+    for name, _, C, _ in bench.LINEARS:
+        w, m = dumps[True][f"{name}.weight.npy"], dumps[True][f"{name}.mask.npy"]
+        assert w.dtype == m.dtype == np.float32 and w.shape == m.shape == (bench.DUMP_ROWS, C)
+        assert set(np.unique(m)) == {0.0, 1.0} and (m.reshape(bench.DUMP_ROWS, -1, 4).sum(axis=2) == 2).all(), name
+        assert (w[m == 0] == 0).all() and (w[m == 1] != 0).mean() > 0.99, name
+    for f in dumps[True]:
+        assert np.array_equal(dumps[True][f], dumps[False][f]), f
+
+
 def test_statistics_roofline_is_quoted_on_distinct_bytes_when_batched(monkeypatch):
     """SURVEY 8(d) asks to say which byte count the roofline uses: with the block's statistics as ONE launch the linears fed
     the same activations share them through L2, so `achieved` / `frac` count the four distinct tensors (12.21 of the 18.66 GB)
