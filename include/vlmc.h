@@ -46,8 +46,9 @@ enum vlmc_status {
   /* numerical status BITS of the factorisation's device status word (0 = clean) */
   VLMC_NOT_POSDEF = 1,        /* Cholesky met a non-positive / NaN pivot (caller damps, retries)           */
   VLMC_NONFINITE = 2,         /* the input matrix holds +-inf or NaN (caller clamps like :101-109, retries) */
-  VLMC_HUGE_FACTOR = 4        /* an entry of U exceeds 1e15: diag(H^-1) may overflow fp32, the caller runs the
+  VLMC_HUGE_FACTOR = 4,       /* an entry of U exceeds 1e15: diag(H^-1) may overflow fp32, the caller runs the
                                  reference's second stage (:131-157) explicitly                           */
+  VLMC_NOT_2OF4 = 8           /* vlmc_sparse24_compress: a group of 4 columns holds more than two non-zeros */
 };
 
 #define VLMC_WS_COUNTER_BYTES 4096
@@ -60,7 +61,8 @@ enum vlmc_op {
   VLMC_OP_HESSIAN = 4,      /* (T, C, 0)       */
   VLMC_OP_CHOL = 5,         /* (C, 0, 0)       */
   VLMC_OP_OBS = 6,          /* (R, C, blocksize) */
-  VLMC_OP_DSNOT_REFINE = 7  /* (R, C, max_cycle_time) */
+  VLMC_OP_DSNOT_REFINE = 7, /* (R, C, max_cycle_time) */
+  VLMC_OP_SPARSE24_LINEAR = 8 /* (T, R, C)       */
 };
 
 int vlmc_version(void);
@@ -265,6 +267,42 @@ size_t vlmc_sparselora_lora_grads_workspace_bytes(int R, int C, int rank);
 int vlmc_sparselora_lora_grads(const void* G, int dtype, int R, int C, int64_t ldg, const uint8_t* keep_mask,
                                int64_t ldm, int sparse, const float* A, const float* B, int rank, float scaling,
                                float* dA, float* dB, void* ws, size_t ws_bytes, void* stream);
+
+/*
+ * Compressed 2:4 weights (K24-K26).  A weight W [R, C] (fp16 / bf16, C % 16 == 0) whose every group of 4 consecutive
+ * columns holds at most two non-zeros - what Wanda / SparseGPT / DSnoT leave with prune_n = 2, prune_m = 4 - is stored as
+ *   values [R, C/2]   W's dtype.  Group g (columns 4g..4g+3) keeps its two values at [2g, 2g+1], in ascending column order.
+ *   meta   [R, C/16]  uint16.  Word j covers columns [16j, 16j+16); group g of the word uses bits [4g, 4g+4): the low
+ *                     2 bits hold the index (0-3) of the first kept element, the high 2 bits the index of the second,
+ *                     first < second.
+ * 0.5625x the bytes of the dense weight.  This is the logical order of NVIDIA's 2:4 metadata, not the interleaved order
+ * the sparse tensor-core instructions read.  The rules that make the format exact and deterministic:
+ *   - an element is kept when w != 0: NaN is kept, +0 and -0 are pruned;
+ *   - a group with fewer than two kept elements is padded with its lowest-index pruned positions, whose stored value is
+ *     +0 (so every group names two distinct indices);
+ *   - a group with more than two non-zeros is rejected: the status word gets VLMC_NOT_2OF4, W is not modified and
+ *     values / meta are unspecified;
+ *   - decompression writes +0 at pruned positions.  A round trip is exact at every non-zero; the only thing not kept is
+ *     the sign of pruned zeros (a pruner that multiplies by the mask leaves -0 where the weight was negative).
+ *
+ * K24  vlmc_sparse24_compress    W -> values, meta.  *status (device int) is cleared, then set to VLMC_NOT_2OF4 if any
+ *                                group is rejected (the call itself returns 0: it does not synchronise).
+ * K25  vlmc_sparse24_decompress  values, meta -> W [R, ldw] (the pruned positions of W are written, +0).
+ * K26  vlmc_sparse24_linear_forward  y[T, R] = x[T, C] . W^T (+ bias[R]) read from the compressed weight: each 128 x 128
+ *                                weight slice is expanded on chip into the dense tensor-core operand (bit-identical to
+ *                                K25's output) and multiplied with tcgen05 (kind::f16, fp32 accumulation).  x, values,
+ *                                bias and y share `dtype`; bias may be NULL; y is rounded once, after the bias.  Small T
+ *                                is split over K: fp32 partials in ws, summed in split order by the tile's last CTA, so
+ *                                equal inputs give equal bits.  ws of vlmc_workspace_bytes(VLMC_OP_SPARSE24_LINEAR, T, R,
+ *                                C).  TMA: ldx, ldv, ldm multiples of 8 elements, x / values / meta 16-byte aligned.
+ */
+int vlmc_sparse24_compress(const void* W, int dtype, int R, int C, int64_t ldw, void* values, int64_t ldv,
+                           uint16_t* meta, int64_t ldm, int* status, void* stream);
+int vlmc_sparse24_decompress(const void* values, int dtype, int R, int C, int64_t ldv, const uint16_t* meta,
+                             int64_t ldm, void* W, int64_t ldw, void* stream);
+int vlmc_sparse24_linear_forward(const void* x, int dtype, int64_t T, int C, int64_t ldx, const void* values,
+                                 int64_t ldv, const uint16_t* meta, int64_t ldm, int R, const void* bias, void* y,
+                                 int64_t ldy, void* ws, size_t ws_bytes, void* stream);
 
 /*
  * K17  Non-zero element counts of up to 64 tensors of one dtype per call ("Remaining Proportion",

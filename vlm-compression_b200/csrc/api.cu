@@ -8,6 +8,7 @@ size_t threshold_workspace_bytes(int R, int C);
 size_t chol_workspace_bytes(int C);
 size_t obs_workspace_bytes(int R, int C);
 size_t dsnot_refine_workspace_bytes(int R, int C, int max_cycle);
+size_t sparse24_linear_workspace_bytes(int64_t T, int R, int C);
 }  // namespace vlmc
 
 extern "C" int vlmc_version(void) { return VLMC_ABI_VERSION; }
@@ -23,6 +24,7 @@ extern "C" const char* vlmc_status_string(int s) {
     case VLMC_ERR_WORKSPACE: return "workspace too small";
     case VLMC_ERR_CUDA: return "CUDA launch failed";
     case VLMC_NOT_POSDEF: return "matrix is not positive definite";
+    case VLMC_NOT_2OF4: return "weight is not 2:4 sparse (a group of 4 columns holds more than two non-zeros)";
     default: return "unknown status";
   }
 }
@@ -44,6 +46,7 @@ extern "C" size_t vlmc_workspace_bytes(int op, int64_t d0, int64_t d1, int64_t d
     case VLMC_OP_CHOL: return chol_workspace_bytes((int)d0);
     case VLMC_OP_OBS: return obs_workspace_bytes((int)d0, (int)d1);
     case VLMC_OP_DSNOT_REFINE: return dsnot_refine_workspace_bytes((int)d0, (int)d1, (int)d2);
+    case VLMC_OP_SPARSE24_LINEAR: return sparse24_linear_workspace_bytes(d0, (int)d1, (int)d2);
     default: return 0;
   }
 }

@@ -11,17 +11,24 @@ Mirrors evaluate_old.py:
   load_pruned_vision_model    <- :268-290   "visual." / "visual_encoder." prefix, missing keys keep the current weights
 The format is the reference's (dense tensors with explicit zeros): checkpoints written here load in evaluate_old.py and
 the other way round.  torch.save / torch.load / yaml are plumbing; the only arithmetic is the non-zero count (K17).
+
+save_compressed_checkpoint / load_compressed_checkpoint write and read a model whose 2:4 linears are compressed
+(vlmc.sparse24): {"format": COMPRESSED_FORMAT, "state_dict": ..., "sparse24": {linear name: in_features}}, the linears'
+entries being `values` / `meta` / `bias` instead of `weight` / `bias`.
 """
 import os
 import time
 
 import torch
+import torch.nn as nn
 import yaml
 
 from vlmc import native
+from vlmc.sparse24 import Sparse24Linear
 
 LANGUAGE_PREFIXES = ("t5_model", "opt_model", "llm_model")      # evaluate_old.py:246,253,260 (checked in this order)
 VISION_PREFIXES = ("visual.", "visual_encoder.")                 # evaluate_old.py:271
+COMPRESSED_FORMAT = "vlmc-sparse24-v1"
 
 
 def remaining_proportion(model, orig_total_size=None):
@@ -91,3 +98,39 @@ def load_pruned_vision_model(model, checkpoint, interpolate_pos_embed=None):
         interpolate_pos_embed(model.visual_encoder, merged)
     model.visual_encoder.load_state_dict(merged)
     return prefix
+
+
+def save_compressed_checkpoint(model, path):
+    """Writes the state of a model whose 2:4 linears are Sparse24Linear (vlmc.sparse24.compress_model) to `path`."""
+    layers = {name: mod.in_features for name, mod in model.named_modules() if isinstance(mod, Sparse24Linear)}
+    state = {k: v.contiguous() for k, v in model.state_dict().items()}
+    torch.save({"format": COMPRESSED_FORMAT, "state_dict": state, "sparse24": layers}, path)
+
+
+def load_compressed_checkpoint(model, path, dense=False):
+    """Loads a file of save_compressed_checkpoint into `model` (dense or already compressed, same architecture).
+    dense=False: the compressed linears become Sparse24Linear (nn.Linears at those names are replaced, on their device).
+    dense=True: the weights are expanded (K25, +0 at pruned positions) into the model's nn.Linears, which stay dense, so
+    the result is an ordinary dense state that the reference's loaders take.  Returns the compressed linears' names."""
+    ckpt = torch.load(path, map_location="cpu")
+    if not isinstance(ckpt, dict) or ckpt.get("format") != COMPRESSED_FORMAT:
+        raise ValueError(f"{path} is not a {COMPRESSED_FORMAT} checkpoint")
+    state, layers = dict(ckpt["state_dict"]), ckpt["sparse24"]
+    for name, C in layers.items():
+        mod = model.get_submodule(name)
+        values, meta = state.pop(name + ".values"), state.pop(name + ".meta")
+        bias = state.get(name + ".bias")
+        ref = mod.weight if isinstance(mod, nn.Linear) else mod.values
+        dev = ref.device if ref.is_cuda else torch.device("cuda")
+        if dense:
+            if not isinstance(mod, nn.Linear):
+                raise TypeError(f"dense=True needs an nn.Linear at {name}, found {type(mod).__name__}")
+            state[name + ".weight"] = native.sparse24_decompress(values.to(dev), meta.to(dev), C)
+            continue
+        if isinstance(mod, nn.Linear):
+            new = Sparse24Linear(values.to(dev), meta.to(dev), C, None if bias is None else bias.to(dev))
+            parent_name, _, child = name.rpartition(".")
+            setattr(model.get_submodule(parent_name) if parent_name else model, child, new)
+        state[name + ".values"], state[name + ".meta"] = values, meta
+    model.load_state_dict(state)
+    return list(layers)

@@ -15,7 +15,8 @@ _LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "lib
 F32, F16, BF16 = 0, 1, 2
 _DTYPES = {torch.float32: F32, torch.float16: F16, torch.bfloat16: BF16}
 
-OP_SQNORM, OP_DSNOT_STATS, OP_WANDA_SELECT, OP_LORA_MERGE, OP_HESSIAN, OP_CHOL, OP_OBS, OP_DSNOT_REFINE = range(8)
+(OP_SQNORM, OP_DSNOT_STATS, OP_WANDA_SELECT, OP_LORA_MERGE, OP_HESSIAN, OP_CHOL, OP_OBS, OP_DSNOT_REFINE,
+ OP_SPARSE24_LINEAR) = range(9)
 WS_COUNTER_BYTES = 4096
 NOT_POSDEF = 1
 
@@ -61,6 +62,9 @@ SIGNATURES = {
     "vlmc_sparselora_linear_forward": (_i, [_vp, _i, _i64, _i, _i64, _vp, _i, _i64, _vp, _vp, _i, _f, _vp, _i64, _i, _vp, _vp, _i64, _vp]),
     "vlmc_sparselora_lora_grads_workspace_bytes": (_sz, [_i, _i, _i]),
     "vlmc_sparselora_lora_grads": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _i, _vp, _vp, _i, _f, _vp, _vp, _vp, _sz, _vp]),
+    "vlmc_sparse24_compress": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _vp, _i64, _vp, _vp]),
+    "vlmc_sparse24_decompress": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _vp, _i64, _vp]),
+    "vlmc_sparse24_linear_forward": (_i, [_vp, _i, _i64, _i, _i64, _vp, _i64, _vp, _i64, _i, _vp, _vp, _i64, _vp, _sz, _vp]),
     "vlmc_count_nonzero_batch": (_i, [_vp, _i, _i, _vp, _vp]),
     "vlmc_scores_workspace_bytes": (_sz, [_vp, _i, _i]),
     "vlmc_scores_kth": (_i, [_vp, _i, _i, _vp, _vp, _vp, _sz, _vp]),
@@ -750,6 +754,114 @@ def sparselora_lora_grads(G, A, B, scaling, keep_mask, sparse=True):
                                             dA.data_ptr(), dB.data_ptr(), ws.data_ptr(), ws.numel(), _stream(G))
     _check("vlmc_sparselora_lora_grads", st)
     return dA, dB
+
+
+NOT_2OF4 = 8                     # status bit of vlmc_sparse24_compress (include/vlmc.h)
+
+
+def _sparse24_weight_dtype(t):
+    if t.dtype not in (torch.float16, torch.bfloat16):
+        raise TypeError(f"compressed 2:4 weights are float16 / bfloat16, got {t.dtype}")
+    return _dtype(t)
+
+
+def _sparse24_operands(values, meta, C):
+    """Checks a (values [R, C/2], meta [R, C/16] int16) pair; meta holds the format's uint16 words bit for bit."""
+    _require_cuda(values, meta)
+    _sparse24_weight_dtype(values)
+    C = int(C)
+    if C < 16 or C % 16:
+        raise ValueError(f"compressed 2:4 weights need C % 16 == 0, got C = {C}")
+    if values.dim() != 2 or values.shape[1] != C // 2 or values.stride(1) != 1:
+        raise ValueError("values must be a row-major [R, C/2] tensor")
+    R = values.shape[0]
+    if meta.dtype != torch.int16 or meta.shape != (R, C // 16) or meta.stride(1) != 1:
+        raise ValueError("meta must be a row-major int16 [R, C/16] tensor")
+    return R, C
+
+
+def sparse24_compress(W):
+    """K24: a 2:4-sparse fp16 / bf16 weight [R, C] -> (values [R, C/2] in W's dtype, meta [R, C/16] int16 holding the
+    uint16 words of include/vlmc.h).  Raises ValueError, leaving W untouched, when a group of 4 columns holds more than
+    two non-zeros (synchronises on the status word)."""
+    _require_cuda(W)
+    dt = _sparse24_weight_dtype(W)
+    if W.dim() != 2 or W.stride(1) != 1:
+        raise ValueError("W must be a 2-D row-major weight")
+    R, C = W.shape
+    if C % 16:
+        raise ValueError(f"compressed 2:4 weights need C % 16 == 0, got C = {C}")
+    values = torch.empty((R, C // 2), dtype=W.dtype, device=W.device)
+    meta = torch.empty((R, C // 16), dtype=torch.int16, device=W.device)
+    status = torch.empty(1, dtype=torch.int32, device=W.device)
+    with torch.cuda.device(W.device):
+        st = load().vlmc_sparse24_compress(W.data_ptr(), dt, R, C, W.stride(0), values.data_ptr(), values.stride(0),
+                                           meta.data_ptr(), meta.stride(0), status.data_ptr(), _stream(W))
+    _check("vlmc_sparse24_compress", st)
+    if int(status.item()) & NOT_2OF4:
+        raise ValueError("weight is not 2:4 sparse: a group of 4 columns holds more than two non-zeros")
+    return values, meta
+
+
+def sparse24_decompress(values, meta, C, out=None):
+    """K25: the dense weight [R, C] of a compressed pair (+0 at pruned positions), into `out` (any row pitch) if given."""
+    R, C = _sparse24_operands(values, meta, C)
+    if out is None:
+        out = torch.empty((R, C), dtype=values.dtype, device=values.device)
+    _require_cuda(out)
+    if out.dtype != values.dtype or out.shape != (R, C) or out.stride(1) != 1:
+        raise ValueError("out must be a row-major [R, C] tensor of the values' dtype")
+    with torch.cuda.device(values.device):
+        st = load().vlmc_sparse24_decompress(values.data_ptr(), _dtype(values), R, C, values.stride(0), meta.data_ptr(),
+                                             meta.stride(0), out.data_ptr(), out.stride(0), _stream(values))
+    _check("vlmc_sparse24_decompress", st)
+    return out
+
+
+def sparse24_linear_supported(x, values, meta, C):
+    """True when K26 takes the call: CUDA tensors, x in the values' fp16 / bf16 dtype, C % 16 == 0, matching shapes."""
+    return (values.is_cuda and meta.is_cuda and x.is_cuda and values.dtype in (torch.float16, torch.bfloat16) and
+            x.dtype == values.dtype and C >= 16 and C % 16 == 0 and x.shape[-1] == C and values.dim() == 2 and
+            values.shape[1] == C // 2 and meta.dtype == torch.int16 and meta.shape == (values.shape[0], C // 16))
+
+
+def sparse24_linear(x, values, meta, C, bias=None, out=None):
+    """K26: y = F.linear(x, decompress(values, meta), bias) read from the compressed weight.  x [..., C] in the values'
+    dtype; returns y [..., R].  Operands whose row pitch TMA cannot take are copied (meta pitch padded to 16 bytes)."""
+    R, C = _sparse24_operands(values, meta, C)
+    _require_cuda(x)
+    if x.dtype != values.dtype or x.shape[-1] != C:
+        raise ValueError("x must be [..., C] in the layer's dtype")
+    x2 = x.reshape(-1, C)
+    if x2.stride(1) != 1 or x2.stride(0) % 8 != 0 or x2.data_ptr() % 16 != 0:
+        x2 = x2.contiguous()
+    if values.stride(0) % 8 != 0 or values.data_ptr() % 16 != 0:
+        values = values.contiguous()
+    if meta.stride(0) % 8 != 0 or meta.data_ptr() % 16 != 0:
+        padded = torch.zeros((R, (C // 16 + 7) // 8 * 8), dtype=torch.int16, device=meta.device)
+        padded[:, :C // 16] = meta
+        meta = padded[:, :C // 16]
+    if bias is not None:
+        _require_cuda(bias)
+        bias = bias.to(values.dtype).contiguous()
+        if bias.shape != (R,):
+            raise ValueError("bias must be [R]")
+    Tn = x2.shape[0]
+    y = out if out is not None else torch.empty((Tn, R), dtype=values.dtype, device=values.device)
+    _require_cuda(y)
+    if y.dtype != values.dtype or y.shape != (Tn, R) or y.stride(1) != 1:
+        raise ValueError("out must be a row-major [T, R] tensor of the values' dtype")
+    if Tn == 0:
+        return y.reshape(*x.shape[:-1], R)
+    lib = load()
+    ws = workspace(x2, lib.vlmc_workspace_bytes(OP_SPARSE24_LINEAR, Tn, R, C))
+    with torch.cuda.device(values.device):
+        st = lib.vlmc_sparse24_linear_forward(x2.data_ptr(), _dtype(values), Tn, C, x2.stride(0), values.data_ptr(),
+                                              values.stride(0), meta.data_ptr(), meta.stride(0), R,
+                                              bias.data_ptr() if bias is not None else None, y.data_ptr(), y.stride(0),
+                                              ws.data_ptr(), ws.numel(), _stream(values))
+    _check("vlmc_sparse24_linear_forward", st)
+    return y.reshape(*x.shape[:-1], R)
 
 
 def hessian_accum(x, H, n_before, b, kc=0, slab_tokens=0):
