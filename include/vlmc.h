@@ -305,6 +305,43 @@ int vlmc_sparse24_linear_forward(const void* x, int dtype, int64_t T, int C, int
                                  int64_t ldy, void* ws, size_t ws_bytes, void* stream);
 
 /*
+ * SparseLoRA on compressed 2:4 weights (K27-K30).  A SparseLoRA layer pruned with lora_model=True keeps its pruned
+ * weights unzeroed and a bool mask beside them, so the kept set cannot come from W's non-zeros.  The mask-driven rule:
+ *   - the kept set IS keep_mask: every group of 4 columns must keep exactly two elements (what Wanda / SparseGPT / DSnoT
+ *     leave with prune_n = 2, prune_m = 4).  Any other count sets VLMC_NOT_2OF4; W is never written;
+ *   - values hold W's bits at the kept positions (+-0, NaN and inf included); there is no padding, so the kept set
+ *     decoded from meta is exactly the mask.
+ * The stored format is the one above, so K25, K26 and the compressed checkpoints read the result unchanged.
+ *
+ * K27  vlmc_sparse24_compress_masked  (W, keep_mask) -> (values, meta).  *status as for K24.  Any pitch and element
+ *                                     alignment of W and keep_mask.
+ * K28  vlmc_sparse24_lora_effective_weight  the weight of the masked training forward (lora.py:364-375) from the
+ *                                     compressed pair: out [R, C] (values' dtype, pitch ldo) bit-identical to
+ *                                     vlmc_sparselora_effective_weight on (decompress(values, meta), mask = meta).
+ * K29  vlmc_sparse24_lora_grads       vlmc_sparselora_lora_grads with the mask read from meta: same results bit for bit,
+ *                                     same workspace (vlmc_sparselora_lora_grads_workspace_bytes).
+ * K30  vlmc_sparse24_lora_merge       Linear.merge() (sparse branch, lora.py:384-394) with the re-mask of
+ *                                     train.py:634-637, in place on values: every stored slot becomes
+ *                                     round(float(v) + scaling * sum_k B A) with K14's arithmetic, so decompress() of
+ *                                     the result equals vlmc_sparselora_merge(remask = 1) on the dense pair.  Only the
+ *                                     sparse branch exists: the dense-delta merge leaves a weight that is not 2:4.
+ * fp16 / bf16, C % 16 == 0, rank <= 16; A = lora_A [rank, C], B = lora_B [R, rank] fp32 row-major, A 16-byte aligned.
+ * K28 / K30: values 8-byte aligned with ldv % 4 == 0; K28's out 16-byte aligned with ldo % 8 == 0.  K29: G 16-byte aligned,
+ * ldg % 8 == 0.  None allocates or retains anything.
+ */
+int vlmc_sparse24_compress_masked(const void* W, int dtype, int R, int C, int64_t ldw, const uint8_t* keep_mask,
+                                  int64_t ldk, void* values, int64_t ldv, uint16_t* meta, int64_t ldm, int* status,
+                                  void* stream);
+int vlmc_sparse24_lora_effective_weight(const void* values, int dtype, int R, int C, int64_t ldv, const uint16_t* meta,
+                                        int64_t ldm, const float* A, const float* B, int rank, float scaling, int sparse,
+                                        void* out, int64_t ldo, void* stream);
+int vlmc_sparse24_lora_grads(const void* G, int dtype, int R, int C, int64_t ldg, const uint16_t* meta, int64_t ldm,
+                             int sparse, const float* A, const float* B, int rank, float scaling, float* dA, float* dB,
+                             void* ws, size_t ws_bytes, void* stream);
+int vlmc_sparse24_lora_merge(void* values, int dtype, int R, int C, int64_t ldv, const uint16_t* meta, int64_t ldm,
+                             const float* A, const float* B, int rank, float scaling, void* stream);
+
+/*
  * K17  Non-zero element counts of up to 64 tensors of one dtype per call ("Remaining Proportion",
  * evaluate_old.py:331-334: sum((param != 0).float().sum() for param in model.parameters())).  `items` is a HOST array
  * read during the call; out[i] (device, uint64) receives the count of items[i].  x != 0 as torch evaluates it (-0.0 is

@@ -11,8 +11,10 @@
 //   K16  vlmc_sparselora_lora_grads         dB = E A^T and dA = B^T E with E = (G (.) mask) * scaling rounded like the
 //                                           reference's backward (W dtype, then fp32): one read of G + mask per output,
 //                                           fp32 accumulation in a fixed order (deterministic)
+//   K29  vlmc_sparse24_lora_grads           K16 with the mask taken from a compressed 2:4 weight's meta (4.25 B / weight)
 // The two dense GEMMs of the step (y = x W_eff^T, G = dy^T x) stay library GEMMs (cuBLAS through torch).
 #include "lora_tile.cuh"
+#include "sparse24.cuh"
 
 namespace vlmc {
 
@@ -65,12 +67,29 @@ __device__ __forceinline__ void grad_e(const uint4& gv, const uint32_t (&mb)[2],
   }
 }
 
+// Where the kernels read the mask of row `row`, columns [col, col + V), as mask bytes: a bool mask (K16) or the meta of
+// a compressed 2:4 weight whose kept set is the mask (K29; sparse24.cuh).  Everything else is the same code.
+struct MaskBytes {
+  const uint8_t* p; int64_t ld;
+  template <int V> __device__ __forceinline__ void load(int row, int col, uint32_t (&mb)[2]) const {
+    const uint8_t* mp = p + (int64_t)row * ld + col;
+    if (V == 8) { const uint2 t = *reinterpret_cast<const uint2*>(mp); mb[0] = t.x; mb[1] = t.y; }
+    else mb[0] = *reinterpret_cast<const uint32_t*>(mp);
+  }
+};
+struct MaskMeta24 {
+  const uint16_t* p; int64_t ld;
+  template <int V> __device__ __forceinline__ void load(int row, int col, uint32_t (&mb)[2]) const {
+    sp_meta_mask<V>(p, ld, row, col, mb);
+  }
+};
+
 // dB[i][k] = sum_j E[i][j] A[k][j]: one warp per row, lanes stride the 16-byte vectors of the row, fixed-order warp
 // reduction.  A (rank x C fp32) is read through L1 / L2 (32-128 KB, shared by every row).
-template <typename T, int RK>
+template <typename T, int RK, class Mask>
 __global__ void __launch_bounds__(256)
-lora_grad_b_kernel(const T* __restrict__ G, int64_t ldg, int R, int C, const uint8_t* __restrict__ mask, int64_t ldm,
-                   int sparse, const float* __restrict__ A, int rank, float scaling, float* __restrict__ dB) {
+lora_grad_b_kernel(const T* __restrict__ G, int64_t ldg, int R, int C, const Mask mask, int sparse,
+                   const float* __restrict__ A, int rank, float scaling, float* __restrict__ dB) {
   constexpr int V = Elem<T>::kVec;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int nvec = C / V;
@@ -81,11 +100,7 @@ lora_grad_b_kernel(const T* __restrict__ G, int64_t ldg, int R, int C, const uin
     for (int j = lane; j < nvec; j += 32) {
       const uint4 gv = ld_stream(G + (int64_t)row * ldg + j * V);
       uint32_t mb[2] = {0x01010101u, 0x01010101u};
-      if (sparse) {
-        const uint8_t* mp = mask + (int64_t)row * ldm + j * V;
-        if (V == 8) { const uint2 t = *reinterpret_cast<const uint2*>(mp); mb[0] = t.x; mb[1] = t.y; }
-        else mb[0] = *reinterpret_cast<const uint32_t*>(mp);
-      }
+      if (sparse) mask.template load<V>(row, j * V, mb);
       float e[V];
       grad_e<T>(gv, mb, sparse, scaling, e);
 #pragma unroll
@@ -113,11 +128,11 @@ lora_grad_b_kernel(const T* __restrict__ G, int64_t ldg, int R, int C, const uin
 
 // dA[k][j] = sum_i B[i][k] E[i][j]: a thread owns 16 bytes of columns, CTAs split the rows into chunks, partial sums
 // go to the workspace [chunk][rank][C] and a second kernel adds the chunks in order.
-template <typename T, int RK>
+template <typename T, int RK, class Mask>
 __global__ void __launch_bounds__(kFwdThreads)
-lora_grad_a_partial_kernel(const T* __restrict__ G, int64_t ldg, int R, int C, const uint8_t* __restrict__ mask,
-                           int64_t ldm, int sparse, const float* __restrict__ B, int rank, float scaling,
-                           int rows_per_chunk, float* __restrict__ part) {
+lora_grad_a_partial_kernel(const T* __restrict__ G, int64_t ldg, int R, int C, const Mask mask, int sparse,
+                           const float* __restrict__ B, int rank, float scaling, int rows_per_chunk,
+                           float* __restrict__ part) {
   constexpr int V = Elem<T>::kVec;
   const int col = (blockIdx.x * kFwdThreads + threadIdx.x) * V;
   if (col >= C) return;
@@ -131,11 +146,7 @@ lora_grad_a_partial_kernel(const T* __restrict__ G, int64_t ldg, int R, int C, c
   for (int row = r0; row < r1; ++row) {
     const uint4 gv = ld_stream(G + (int64_t)row * ldg + col);
     uint32_t mb[2] = {0x01010101u, 0x01010101u};
-    if (sparse) {
-      const uint8_t* mp = mask + (int64_t)row * ldm + col;
-      if (V == 8) { const uint2 t = *reinterpret_cast<const uint2*>(mp); mb[0] = t.x; mb[1] = t.y; }
-      else mb[0] = *reinterpret_cast<const uint32_t*>(mp);
-    }
+    if (sparse) mask.template load<V>(row, col, mb);
     float e[V];
     grad_e<T>(gv, mb, sparse, scaling, e);
     const float* brow = B + (int64_t)row * rank;
@@ -172,6 +183,35 @@ static int grad_chunks(int R) {
   int chunks = kNumSMs * 2;                 // with C / (128 * V) column tiles this fills the GPU for every shape on the path
   if (chunks > (R + 15) / 16) chunks = (R + 15) / 16;
   return chunks < 1 ? 1 : chunks;
+}
+
+// the launches of K16 / K29 (the mask source is the only difference): dB, the dA partials, the ordered chunk sum
+template <class Mask>
+static int lora_grads_launch(const void* G, int dtype, int R, int C, int64_t ldg, const Mask mask, int sparse,
+                             const float* A, const float* B, int rank, float scaling, float* dA, float* dB, void* ws,
+                             cudaStream_t st) {
+  const int V = dtype == VLMC_F32 ? 4 : 8;
+  float* part = reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + VLMC_WS_COUNTER_BYTES);
+  int bgrid = (R + 7) / 8;
+  if (bgrid > kNumSMs * 8) bgrid = kNumSMs * 8;
+  const int chunks = grad_chunks(R);
+  const int rows_per_chunk = (R + chunks - 1) / chunks;
+  const int nchunks = (R + rows_per_chunk - 1) / rows_per_chunk;
+  dim3 agrid((C / V + kFwdThreads - 1) / kFwdThreads, nchunks);
+#define VLMC_GRADS(RK)                                                                                                  \
+  VLMC_DISPATCH_DTYPE(dtype, {                                                                                          \
+    lora_grad_b_kernel<scalar_t, RK, Mask><<<bgrid, 256, 0, st>>>(reinterpret_cast<const scalar_t*>(G), ldg, R, C,     \
+                                                                  mask, sparse, A, rank, scaling, dB);                  \
+    lora_grad_a_partial_kernel<scalar_t, RK, Mask><<<agrid, kFwdThreads, 0, st>>>(                                      \
+        reinterpret_cast<const scalar_t*>(G), ldg, R, C, mask, sparse, B, rank, scaling, rows_per_chunk, part);         \
+  })
+  if (rank <= 4) { VLMC_GRADS(4); }
+  else if (rank <= 8) { VLMC_GRADS(8); }
+  else { VLMC_GRADS(16); }
+#undef VLMC_GRADS
+  const int64_t n = (int64_t)rank * C;
+  lora_grad_a_reduce_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(part, nchunks, n, dA);
+  return check_launch();
 }
 
 }  // namespace vlmc
@@ -236,26 +276,25 @@ extern "C" int vlmc_sparselora_lora_grads(const void* G, int dtype, int R, int C
       !is_device_ptr(ws) || (sparse && !is_device_ptr(keep_mask)))
     return VLMC_ERR_NOT_DEVICE;
   if (ws_bytes < vlmc_sparselora_lora_grads_workspace_bytes(R, C, rank)) return VLMC_ERR_WORKSPACE;
-  cudaStream_t st = (cudaStream_t)stream;
-  float* part = reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + VLMC_WS_COUNTER_BYTES);
-  int bgrid = (R + 7) / 8;
-  if (bgrid > kNumSMs * 8) bgrid = kNumSMs * 8;
-  const int chunks = grad_chunks(R);
-  const int rows_per_chunk = (R + chunks - 1) / chunks;
-  const int nchunks = (R + rows_per_chunk - 1) / rows_per_chunk;
-  dim3 agrid((C / V + kFwdThreads - 1) / kFwdThreads, nchunks);
-#define VLMC_GRADS(RK)                                                                                                  \
-  VLMC_DISPATCH_DTYPE(dtype, {                                                                                          \
-    lora_grad_b_kernel<scalar_t, RK><<<bgrid, 256, 0, st>>>(reinterpret_cast<const scalar_t*>(G), ldg, R, C, keep_mask, \
-                                                            ldm, sparse, A, rank, scaling, dB);                         \
-    lora_grad_a_partial_kernel<scalar_t, RK><<<agrid, kFwdThreads, 0, st>>>(                                            \
-        reinterpret_cast<const scalar_t*>(G), ldg, R, C, keep_mask, ldm, sparse, B, rank, scaling, rows_per_chunk, part); \
-  })
-  if (rank <= 4) { VLMC_GRADS(4); }
-  else if (rank <= 8) { VLMC_GRADS(8); }
-  else { VLMC_GRADS(16); }
-#undef VLMC_GRADS
-  const int64_t n = (int64_t)rank * C;
-  lora_grad_a_reduce_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(part, nchunks, n, dA);
-  return check_launch();
+  return lora_grads_launch(G, dtype, R, C, ldg, MaskBytes{keep_mask, ldm}, sparse, A, B, rank, scaling, dA, dB, ws,
+                           (cudaStream_t)stream);
+}
+
+// K29: K16 with the mask read from the meta of a mask-driven compressed 2:4 weight (K27), same kernels and workspace
+extern "C" int vlmc_sparse24_lora_grads(const void* G, int dtype, int R, int C, int64_t ldg, const uint16_t* meta,
+                                        int64_t ldm, int sparse, const float* A, const float* B, int rank, float scaling,
+                                        float* dA, float* dB, void* ws, size_t ws_bytes, void* stream) {
+  using namespace vlmc;
+  if (!G || !A || !B || !dA || !dB || !ws || R < 1 || C < 16 || rank < 1 || ldg < C) return VLMC_ERR_BAD_ARG;
+  if (sparse && (!meta || ldm < C / 16)) return VLMC_ERR_BAD_ARG;
+  if (dtype != VLMC_F16 && dtype != VLMC_BF16) return dtype == VLMC_F32 ? VLMC_ERR_UNSUPPORTED : VLMC_ERR_BAD_ARG;
+  if (rank > kGradMaxRank) return VLMC_ERR_UNSUPPORTED;
+  if (C % 16 != 0 || ldg % 8 != 0 || ((uintptr_t)G & 15) != 0 || ((uintptr_t)A & 15) != 0 || ((uintptr_t)meta & 1) != 0)
+    return VLMC_ERR_UNSUPPORTED;
+  if (!is_device_ptr(G) || !is_device_ptr(A) || !is_device_ptr(B) || !is_device_ptr(dA) || !is_device_ptr(dB) ||
+      !is_device_ptr(ws) || (sparse && !is_device_ptr(meta)))
+    return VLMC_ERR_NOT_DEVICE;
+  if (ws_bytes < vlmc_sparselora_lora_grads_workspace_bytes(R, C, rank)) return VLMC_ERR_WORKSPACE;
+  return lora_grads_launch(G, dtype, R, C, ldg, MaskMeta24{meta, ldm}, sparse, A, B, rank, scaling, dA, dB, ws,
+                           (cudaStream_t)stream);
 }

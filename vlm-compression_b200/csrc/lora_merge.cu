@@ -50,16 +50,7 @@ lora_merge_batch_kernel(const __grid_constant__ MergeBatch b, int remask) {
     const float scaling = it.scaling;
     T* W = reinterpret_cast<T*>(it.W);
     lt_rows<T>(W, it.ldw, W, it.ldw, col, rb * kLtUnitRows, row_end, it.B, it.rank, it.mask, it.ldm, lt_sA,
-               [&](float (&f)[V], const float (&acc)[V], const uint32_t (&mb)[2]) {
-#pragma unroll
-                 for (int e = 0; e < V; ++e) {
-                   const bool keep = (mb[e / 4] >> (8 * (e % 4))) & 0xffu;
-                   // (BA * scaling) * mask, then W += : two separately rounded fp32 ops, no FMA contraction
-                   const float delta = __fmul_rn(acc[e], scaling);
-                   const float merged = __fadd_rn(f[e], delta);
-                   f[e] = keep ? merged : (remask ? 0.f : f[e]);
-                 }
-               });
+               [&](float (&f)[V], const float (&acc)[V], const uint32_t (&mb)[2]) { lt_merge<T>(f, acc, mb, scaling, remask); });
   }
 }
 

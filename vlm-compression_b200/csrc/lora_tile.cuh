@@ -1,4 +1,5 @@
-// The streaming tile loop K14 (masked merge, in place) and K15 (effective weight, out of place) share.
+// The streaming tile loop K14 (masked merge, in place) and K15 (effective weight, out of place) share; sparse24.cuh holds
+// its compressed-weight variant (K28, K30).
 //
 // A 128-thread CTA walks a contiguous span of units of kLtUnitRows rows x 1024 columns (16 bytes of W per thread and row).
 // The rank x 1024 slice of lora_A it needs is staged in shared memory when the span enters a new column tile (once or twice per CTA) as float4 planes (conflict-free 16-byte reads), so a
@@ -75,6 +76,56 @@ __device__ __forceinline__ void lt_stage_a(float4* sA, const float* __restrict__
     }
 }
 
+// K14's combine (lora.py:384-387 + train.py:634-637): f[V] <- keep ? round(W + (BA * scaling)) : (remask ? 0 : W), the
+// rounding to W's dtype left to the store.  (BA * scaling) * mask, then W += : two separately rounded fp32 ops, no FMA
+// contraction.  Shared by the dense merge (K14) and the compressed one (K30).
+template <typename T, int V = Elem<T>::kVec>
+__device__ __forceinline__ void lt_merge(float (&f)[V], const float (&acc)[V], const uint32_t (&mb)[2], float scaling,
+                                         int remask) {
+#pragma unroll
+  for (int e = 0; e < V; ++e) {
+    const bool keep = (mb[e / 4] >> (8 * (e % 4))) & 0xffu;
+    const float delta = __fmul_rn(acc[e], scaling);
+    const float merged = __fadd_rn(f[e], delta);
+    f[e] = keep ? merged : (remask ? 0.f : f[e]);
+  }
+}
+
+// acc[r][.] = sum_k B[row0 + r][k] A[k][this thread's V columns] for the kLtRows rows from row0 (rows past row_end repeat
+// the last row and are not stored).  The rank-r dot on packed fp32 FMAs (fma.rn.f32x2, sm_100): two IEEE fmas per
+// instruction, per lane identical to fmaf - the loop is instruction-issue bound (8 fmas per weight at r = 8), not HBM
+// bound, without them.  k ascending, so every caller gets the same bits for the same (B, A).
+template <typename T>
+__device__ __forceinline__ void lt_dot(float2 (&acc)[kLtRows][Elem<T>::kVec / 2], const float* __restrict__ B, int rank,
+                                       int row0, int row_end, const float4* sA) {
+  constexpr int V = Elem<T>::kVec;
+  const int t = threadIdx.x;
+#pragma unroll
+  for (int r = 0; r < kLtRows; ++r)
+#pragma unroll
+    for (int e = 0; e < V / 2; ++e) acc[r][e] = make_float2(0.f, 0.f);
+  const float* brow[kLtRows];
+#pragma unroll
+  for (int r = 0; r < kLtRows; ++r) brow[r] = B + (int64_t)(row0 + r < row_end ? row0 + r : row_end - 1) * rank;
+#pragma unroll 4
+  for (int kk = 0; kk < rank; ++kk) {
+    float2 a[V / 2];
+#pragma unroll
+    for (int q = 0; q < V / 4; ++q) {
+      const float4 av = sA[(kk * (V / 4) + q) * kLtThreads + t];
+      a[2 * q] = make_float2(av.x, av.y);
+      a[2 * q + 1] = make_float2(av.z, av.w);
+    }
+#pragma unroll
+    for (int r = 0; r < kLtRows; ++r) {
+      const float b = __ldg(brow[r] + kk);
+      const float2 b2 = make_float2(b, b);
+#pragma unroll
+      for (int e = 0; e < V / 2; ++e) acc[r][e] = __ffma2_rn(b2, a[e], acc[r][e]);      // k ascending, like SGEMM
+    }
+  }
+}
+
 // rows [row_begin, row_end) of this thread's 16-byte column.  comb(f, acc, mb) rewrites f[V] from the weights f, the
 // rank-r dot acc = sum_k B[row][k] A[k][col..] and the mask bytes mb, then the vector is stored to out.
 template <typename T, class Combine>
@@ -82,7 +133,6 @@ __device__ __forceinline__ void lt_rows(const T* __restrict__ W, int64_t ldw, T*
                                         int row_begin, int row_end, const float* __restrict__ B, int rank,
                                         const uint8_t* __restrict__ mask, int64_t ldm, const float4* sA, Combine comb) {
   constexpr int V = Elem<T>::kVec;
-  const int t = threadIdx.x;
   for (int row0 = row_begin; row0 < row_end; row0 += kLtRows) {
     uint4 wv[kLtRows];
     uint2 mv[kLtRows];
@@ -95,33 +145,8 @@ __device__ __forceinline__ void lt_rows(const T* __restrict__ W, int64_t ldw, T*
         else mv[r] = make_uint2(*reinterpret_cast<const uint32_t*>(mp), 0u);
       }
     }
-    // the rank-r dot on packed fp32 FMAs (fma.rn.f32x2, sm_100): two IEEE fmas per instruction, per lane identical to
-    // fmaf - the loop is instruction-issue bound (8 fmas per weight at r = 8), not HBM bound, without them
     float2 acc[kLtRows][V / 2];
-#pragma unroll
-    for (int r = 0; r < kLtRows; ++r)
-#pragma unroll
-      for (int e = 0; e < V / 2; ++e) acc[r][e] = make_float2(0.f, 0.f);
-    const float* brow[kLtRows];
-#pragma unroll
-    for (int r = 0; r < kLtRows; ++r) brow[r] = B + (int64_t)(row0 + r < row_end ? row0 + r : row_end - 1) * rank;
-#pragma unroll 4
-    for (int kk = 0; kk < rank; ++kk) {
-      float2 a[V / 2];
-#pragma unroll
-      for (int q = 0; q < V / 4; ++q) {
-        const float4 av = sA[(kk * (V / 4) + q) * kLtThreads + t];
-        a[2 * q] = make_float2(av.x, av.y);
-        a[2 * q + 1] = make_float2(av.z, av.w);
-      }
-#pragma unroll
-      for (int r = 0; r < kLtRows; ++r) {
-        const float b = __ldg(brow[r] + kk);
-        const float2 b2 = make_float2(b, b);
-#pragma unroll
-        for (int e = 0; e < V / 2; ++e) acc[r][e] = __ffma2_rn(b2, a[e], acc[r][e]);      // k ascending, like SGEMM
-      }
-    }
+    lt_dot<T>(acc, B, rank, row0, row_end, sA);
 #pragma unroll
     for (int r = 0; r < kLtRows; ++r) {
       if (row0 + r >= row_end) break;

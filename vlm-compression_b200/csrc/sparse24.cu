@@ -1,6 +1,8 @@
 // K24-K26: compressed 2:4 weights for pruned models (format: include/vlmc.h, "Compressed 2:4 weights").
 //
 // K24 vlmc_sparse24_compress    W [R, C] -> values [R, C/2] + meta [R, C/16] uint16, one pass, a thread per 16-column word
+// K27 vlmc_sparse24_compress_masked  W + bool mask -> values + meta: the kept set is the mask (SparseLoRA layers keep
+//     their pruned weights unzeroed), exactly two per group
 // K25 vlmc_sparse24_decompress  values + meta -> dense W (+0 at pruned positions); the expand step of the large-T path
 // K26 vlmc_sparse24_linear_forward  y[T, R] = x[T, C] . W^T (+ bias) reading the COMPRESSED weight: 1.125 B per weight of
 //     HBM instead of 2, which is what decode-sized token counts pay for.  Each 128-row x 128-column weight slice is expanded
@@ -16,6 +18,7 @@
 //   warps 7-10   drain: tcgen05.ld -> (+ bias, one rounding) -> y, or fp32 partial -> workspace; the last CTA of a tile
 //                (ticket) sums the partials in split order, so the result does not depend on which CTA finishes last
 #include "tc.cuh"
+#include "sparse24.cuh"
 
 namespace vlmc {
 
@@ -80,12 +83,6 @@ __device__ __forceinline__ uint64_t sp_desc(uint32_t saddr) {
   d |= (uint64_t)1 << 46;
   d |= (uint64_t)2 << 61;
   return d;
-}
-
-// one 4-column group: the value pair (first kept in the low half) and its 4-bit index nibble -> four 16-bit slots
-__device__ __forceinline__ uint64_t sp_expand_group(uint32_t pair, uint32_t nib) {
-  const uint32_t i0 = nib & 3u, i1 = (nib >> 2) & 3u;
-  return ((uint64_t)(pair & 0xffffu) << (16 * i0)) | ((uint64_t)(pair >> 16) << (16 * i1));
 }
 
 template <typename T> __device__ __forceinline__ uint16_t sp_round(float v);
@@ -364,6 +361,68 @@ sparse24_compress_kernel(const uint16_t* __restrict__ W, int64_t ldw, int R, int
   if (__syncthreads_or(bad) && threadIdx.x == 0) atomicOr(status, VLMC_NOT_2OF4);
 }
 
+// K27: the kept set read from a bool mask instead of W's non-zeros.  Exactly two kept per group, else VLMC_NOT_2OF4;
+// the values keep W's bits at the kept positions (+-0, NaN and inf included).
+__device__ __forceinline__ void sp_load16_mask(const uint8_t* src, bool vec, uint32_t* kept4) {
+  uint8_t b[16];
+  if (vec) {
+    const uint4 a = ld_stream(src);
+    const uint32_t w[4] = {a.x, a.y, a.z, a.w};
+#pragma unroll
+    for (int i = 0; i < 16; ++i) b[i] = (uint8_t)(w[i / 4] >> (8 * (i % 4)));
+  } else {
+#pragma unroll
+    for (int i = 0; i < 16; ++i) b[i] = src[i];
+  }
+#pragma unroll
+  for (int g = 0; g < 4; ++g) {
+    uint32_t k = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) k |= (uint32_t)(b[4 * g + i] != 0) << i;
+    kept4[g] = k;
+  }
+}
+
+template <bool kVec>
+__global__ void __launch_bounds__(256)
+sparse24_compress_masked_kernel(const uint16_t* __restrict__ W, int64_t ldw, const uint8_t* __restrict__ mask,
+                                int64_t ldk, int R, int wpr, uint16_t* __restrict__ vals, int64_t ldv,
+                                uint16_t* __restrict__ meta, int64_t ldm, int* status) {
+  const int64_t total = (int64_t)R * wpr;
+  bool bad = false;
+  for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < total; idx += (int64_t)gridDim.x * blockDim.x) {
+    const int r = (int)(idx / wpr), wd = (int)(idx - (int64_t)r * wpr);
+    uint16_t e[16];
+    uint32_t kept[4];
+    sp_load16(W + r * ldw + 16 * wd, kVec, e);
+    sp_load16_mask(mask + r * ldk + 16 * wd, kVec, kept);
+    uint32_t out[4], mw = 0;
+#pragma unroll
+    for (int g = 0; g < 4; ++g) {
+      bad |= __popc(kept[g]) != 2;
+      const uint32_t sel = kept[g] ? kept[g] : 1u;
+      const uint32_t i0 = __ffs(sel) - 1, i1 = 31 - __clz(sel);
+      uint32_t v0 = 0, v1 = 0;
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        v0 = i == (int)i0 ? e[4 * g + i] : v0;
+        v1 = i == (int)i1 ? e[4 * g + i] : v1;
+      }
+      out[g] = v0 | (v1 << 16);
+      mw |= (i0 | (i1 << 2)) << (4 * g);
+    }
+    uint16_t* dv = vals + r * ldv + 8 * wd;
+    if (kVec) {
+      st_stream(dv, make_uint4(out[0], out[1], out[2], out[3]));
+    } else {
+#pragma unroll
+      for (int g = 0; g < 4; ++g) { dv[2 * g] = (uint16_t)out[g]; dv[2 * g + 1] = (uint16_t)(out[g] >> 16); }
+    }
+    meta[r * ldm + wd] = (uint16_t)mw;
+  }
+  if (__syncthreads_or(bad) && threadIdx.x == 0) atomicOr(status, VLMC_NOT_2OF4);
+}
+
 template <bool kVec>
 __global__ void __launch_bounds__(256)
 sparse24_decompress_kernel(const uint16_t* __restrict__ vals, int64_t ldv, const uint16_t* __restrict__ meta, int64_t ldm,
@@ -478,6 +537,30 @@ extern "C" int vlmc_sparse24_compress(const void* W, int dtype, int R, int C, in
   uint16_t* v16 = static_cast<uint16_t*>(values);
   if (vec) sparse24_compress_kernel<true><<<grid, 256, 0, st>>>(w16, ldw, R, wpr, v16, ldv, meta, ldm, status);
   else sparse24_compress_kernel<false><<<grid, 256, 0, st>>>(w16, ldw, R, wpr, v16, ldv, meta, ldm, status);
+  return check_launch();
+}
+
+extern "C" int vlmc_sparse24_compress_masked(const void* W, int dtype, int R, int C, int64_t ldw, const uint8_t* keep_mask,
+                                             int64_t ldk, void* values, int64_t ldv, uint16_t* meta, int64_t ldm, int* status,
+                                             void* stream) {
+  using namespace vlmc;
+  if (!W || !keep_mask || !values || !meta || !status || R < 1 || C < 16 || C % 16 != 0 || ldw < C || ldk < C ||
+      ldv < C / 2 || ldm < C / 16)
+    return VLMC_ERR_BAD_ARG;
+  if (dtype != VLMC_F16 && dtype != VLMC_BF16) return dtype == VLMC_F32 ? VLMC_ERR_UNSUPPORTED : VLMC_ERR_BAD_ARG;
+  if (!is_device_ptr(W) || !is_device_ptr(keep_mask) || !is_device_ptr(values) || !is_device_ptr(meta) ||
+      !is_device_ptr(status))
+    return VLMC_ERR_NOT_DEVICE;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (cudaMemsetAsync(status, 0, sizeof(int), st) != cudaSuccess) return check_launch();
+  const int wpr = C / 16;
+  const bool vec = sp_aligned16(W) && sp_aligned16(values) && sp_aligned16(keep_mask) && ldw % 8 == 0 && ldv % 8 == 0 &&
+                   ldk % 16 == 0;
+  const int grid = sp_grid((int64_t)R * wpr);
+  const uint16_t* w16 = static_cast<const uint16_t*>(W);
+  uint16_t* v16 = static_cast<uint16_t*>(values);
+  if (vec) sparse24_compress_masked_kernel<true><<<grid, 256, 0, st>>>(w16, ldw, keep_mask, ldk, R, wpr, v16, ldv, meta, ldm, status);
+  else sparse24_compress_masked_kernel<false><<<grid, 256, 0, st>>>(w16, ldw, keep_mask, ldk, R, wpr, v16, ldv, meta, ldm, status);
   return check_launch();
 }
 

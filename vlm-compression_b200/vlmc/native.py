@@ -65,6 +65,10 @@ SIGNATURES = {
     "vlmc_sparse24_compress": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _vp, _i64, _vp, _vp]),
     "vlmc_sparse24_decompress": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _vp, _i64, _vp]),
     "vlmc_sparse24_linear_forward": (_i, [_vp, _i, _i64, _i, _i64, _vp, _i64, _vp, _i64, _i, _vp, _vp, _i64, _vp, _sz, _vp]),
+    "vlmc_sparse24_compress_masked": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp]),
+    "vlmc_sparse24_lora_effective_weight": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _vp, _vp, _i, _f, _i, _vp, _i64, _vp]),
+    "vlmc_sparse24_lora_grads": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _i, _vp, _vp, _i, _f, _vp, _vp, _vp, _sz, _vp]),
+    "vlmc_sparse24_lora_merge": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _vp, _vp, _i, _f, _vp]),
     "vlmc_count_nonzero_batch": (_i, [_vp, _i, _i, _vp, _vp]),
     "vlmc_scores_workspace_bytes": (_sz, [_vp, _i, _i]),
     "vlmc_scores_kth": (_i, [_vp, _i, _i, _vp, _vp, _vp, _sz, _vp]),
@@ -1143,3 +1147,104 @@ def dsnot_refine(W, scaler_row, sum_metric_row, var, k, prune_n=0, prune_m=0, po
                                          ws.numel(), _stream(W))
         _check("vlmc_dsnot_refine_apply", st)
     return keep_mask, ncyc
+
+
+def sparse24_compress_masked(W, keep_mask):
+    """K27: (W [R, C] fp16 / bf16, keep_mask [R, C] bool) -> (values [R, C/2], meta [R, C/16] int16) with the kept set
+    read from the mask, not from W's non-zeros: the values keep W's bits at exactly the mask's positions.  Raises
+    ValueError unless every group of 4 columns keeps exactly two (synchronises on the status word).  W is not modified."""
+    _require_cuda(W, keep_mask)
+    dt = _sparse24_weight_dtype(W)
+    if W.dim() != 2 or W.stride(1) != 1:
+        raise ValueError("W must be a 2-D row-major weight")
+    R, C = W.shape
+    if C < 16 or C % 16:
+        raise ValueError(f"compressed 2:4 weights need C % 16 == 0, got C = {C}")
+    if keep_mask.dtype != torch.bool or keep_mask.shape != W.shape or keep_mask.stride(1) != 1:
+        raise ValueError("mask must be a row-major bool tensor shaped like W")
+    values = torch.empty((R, C // 2), dtype=W.dtype, device=W.device)
+    meta = torch.empty((R, C // 16), dtype=torch.int16, device=W.device)
+    status = torch.empty(1, dtype=torch.int32, device=W.device)
+    with torch.cuda.device(W.device):
+        st = load().vlmc_sparse24_compress_masked(W.data_ptr(), dt, R, C, W.stride(0), keep_mask.data_ptr(),
+                                                  keep_mask.stride(0), values.data_ptr(), values.stride(0), meta.data_ptr(),
+                                                  meta.stride(0), status.data_ptr(), _stream(W))
+    _check("vlmc_sparse24_compress_masked", st)
+    if int(status.item()) & NOT_2OF4:
+        raise ValueError("mask is not 2:4: a group of 4 columns does not keep exactly two elements")
+    return values, meta
+
+
+def _sparse24_lora_common(values, meta, C, A, B):
+    R, C = _sparse24_operands(values, meta, C)
+    _require_cuda(A, B)
+    if A.dtype != torch.float32 or B.dtype != torch.float32:
+        raise TypeError("lora_A / lora_B must be float32")
+    rank = A.shape[0]
+    if A.dim() != 2 or A.shape != (rank, C) or B.shape != (R, rank):
+        raise ValueError("lora_A must be [r, C] and lora_B [R, r]")
+    if values.stride(0) % 4 or values.data_ptr() % 8:
+        raise ValueError("values rows must be 8-byte aligned")
+    return R, C, rank, A.contiguous(), B.contiguous()
+
+
+def sparse24_lora_effective_weight(values, meta, C, A, B, scaling, sparse=True, out=None):
+    """K28 (lora.py:364-375) on a mask-driven compressed weight: (W + s*BA) * M or W * M + s*BA with W = decompress(values,
+    meta) and M the kept set of meta, in the values' dtype.  Bit-identical to sparselora_effective_weight on (W, M).
+    Returns `out` [R, C] (any row pitch that keeps 16-byte rows)."""
+    R, C, rank, A, B = _sparse24_lora_common(values, meta, C, A, B)
+    if out is None:
+        out = torch.empty((R, C), dtype=values.dtype, device=values.device)
+    _require_cuda(out)
+    if out.dtype != values.dtype or out.shape != (R, C) or out.stride(1) != 1:
+        raise ValueError("out must be a row-major [R, C] tensor of the values' dtype")
+    with torch.cuda.device(values.device):
+        st = load().vlmc_sparse24_lora_effective_weight(values.data_ptr(), _dtype(values), R, C, values.stride(0),
+                                                        meta.data_ptr(), meta.stride(0), A.data_ptr(), B.data_ptr(), rank,
+                                                        float(scaling), int(bool(sparse)), out.data_ptr(), out.stride(0),
+                                                        _stream(values))
+    _check("vlmc_sparse24_lora_effective_weight", st)
+    return out
+
+
+def sparse24_lora_grads(G, meta, A, B, scaling, sparse=True):
+    """K29: sparselora_lora_grads with the mask taken from meta.  G [R, C] (the values' dtype) -> (dA [r, C], dB [R, r])
+    fp32, bit-identical to K16 on (G, M)."""
+    _require_cuda(G, meta, A, B)
+    _sparse24_weight_dtype(G)
+    if G.dim() != 2 or G.stride(1) != 1:
+        raise ValueError("G must be a 2-D row-major tensor")
+    R, C = G.shape
+    if C < 16 or C % 16:
+        raise ValueError(f"compressed 2:4 weights need C % 16 == 0, got C = {C}")
+    if meta.dtype != torch.int16 or meta.shape != (R, C // 16) or meta.stride(1) != 1:
+        raise ValueError("meta must be a row-major int16 [R, C/16] tensor")
+    if A.dtype != torch.float32 or B.dtype != torch.float32:
+        raise TypeError("lora_A / lora_B must be float32")
+    rank = A.shape[0]
+    if A.shape != (rank, C) or B.shape != (R, rank):
+        raise ValueError("lora_A must be [r, C] and lora_B [R, r]")
+    A, B = A.contiguous(), B.contiguous()
+    lib = load()
+    dA = torch.empty((rank, C), dtype=torch.float32, device=G.device)
+    dB = torch.empty((R, rank), dtype=torch.float32, device=G.device)
+    ws = workspace(G, lib.vlmc_sparselora_lora_grads_workspace_bytes(R, C, rank))
+    with torch.cuda.device(G.device):
+        st = lib.vlmc_sparse24_lora_grads(G.data_ptr(), _dtype(G), R, C, G.stride(0), meta.data_ptr(), meta.stride(0),
+                                          int(bool(sparse)), A.data_ptr(), B.data_ptr(), rank, float(scaling),
+                                          dA.data_ptr(), dB.data_ptr(), ws.data_ptr(), ws.numel(), _stream(G))
+    _check("vlmc_sparse24_lora_grads", st)
+    return dA, dB
+
+
+def sparse24_lora_merge(values, meta, C, A, B, scaling):
+    """K30 (lora.py:384-394 + train.py:634-637), in place on values: every stored slot becomes
+    round(v + s * (B A)[slot]) with K14's arithmetic; decompress() of the result equals sparselora_merge(W, A, B, s, M,
+    remask=True) on the dense pair."""
+    R, C, rank, A, B = _sparse24_lora_common(values, meta, C, A, B)
+    with torch.cuda.device(values.device):
+        st = load().vlmc_sparse24_lora_merge(values.data_ptr(), _dtype(values), R, C, values.stride(0), meta.data_ptr(),
+                                             meta.stride(0), A.data_ptr(), B.data_ptr(), rank, float(scaling),
+                                             _stream(values))
+    _check("vlmc_sparse24_lora_merge", st)
+    return values

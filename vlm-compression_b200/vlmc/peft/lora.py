@@ -35,25 +35,40 @@ def _use_fused(x, W, mask, rank):
     return True
 
 
+class DenseWeightSource:
+    """Where _MaskedLoRALinear gets W_eff and the LoRA gradients for a dense frozen weight W and a bool mask M:
+    K15 and K16.  vlmc.sparse24 has the compressed 2:4 source (K28 / K29), which takes (values, meta) in their place."""
+    fused = True                           # K23 (VLMC_LORA_FUSED=1) reads this form
+
+    @staticmethod
+    def effective_weight(W, mask, A, B, scaling, sparse):
+        return native.sparselora_effective_weight(W, A, B, scaling, mask, sparse)
+
+    @staticmethod
+    def lora_grads(G, mask, A, B, scaling, sparse):
+        return native.sparselora_lora_grads(G, A, B, scaling, mask, sparse)
+
+
 class _MaskedLoRALinear(torch.autograd.Function):
     """y = F.linear(x, W_eff, bias) with W_eff = (W + s*BA) * M (sparse) or W * M + s*BA (lora.py:364-375).
-    W_eff is rebuilt in backward (one K15 pass) instead of being kept alive between forward and backward."""
+    W_eff is rebuilt in backward (one K15 pass) instead of being kept alive between forward and backward.  `source`
+    (DenseWeightSource or a compressed one) says how W and mask are stored."""
 
     # custom_fwd / custom_bwd: backward runs under the autocast state of forward, so with fp32 LoRA'd weights under
     # maybe_autocast(), or fp16 weights under bf16 autocast, gy (autocast dtype) meets w_eff (weight dtype) inside an
     # autocast region exactly like the reference's plain-autograd F.linear does
     @staticmethod
     @torch.amp.custom_fwd(device_type="cuda")
-    def forward(ctx, x, W, A, B, bias, mask, scaling, sparse):
+    def forward(ctx, x, W, A, B, bias, mask, scaling, sparse, source):
         Af, Bf = A.detach().float(), B.detach().float()
         ctx.save_for_backward(x, W, A, B, mask)
-        ctx.scaling, ctx.sparse, ctx.has_bias = scaling, sparse, bias is not None
+        ctx.scaling, ctx.sparse, ctx.has_bias, ctx.source = scaling, sparse, bias is not None, source
         ctx.bias_dtype = bias.dtype if bias is not None else None
-        if _use_fused(x, W, mask, Af.shape[0]):
+        if source.fused and _use_fused(x, W, mask, Af.shape[0]):
             # K23: the effective weight is built on chip, slice by slice, in front of the tensor core - nothing dense is
             # written to HBM.  Same operand bits as K15 (test_lora_linear_fused_operand_is_k15_bit_exact).
             return native.sparselora_linear_forward(x, W.detach(), Af, Bf, scaling, mask, sparse, bias=bias)
-        w_eff = native.sparselora_effective_weight(W.detach(), Af, Bf, scaling, mask, sparse)
+        w_eff = source.effective_weight(W.detach(), mask, Af, Bf, scaling, sparse)
         return F.linear(x, w_eff, bias)
 
     @staticmethod
@@ -64,18 +79,18 @@ class _MaskedLoRALinear(torch.autograd.Function):
         gx = dA = dB = gbias = None
         gy2 = gy.reshape(-1, gy.shape[-1])
         if ctx.needs_input_grad[0]:
-            w_eff = native.sparselora_effective_weight(W.detach(), Af, Bf, ctx.scaling, mask, ctx.sparse)
+            w_eff = ctx.source.effective_weight(W.detach(), mask, Af, Bf, ctx.scaling, ctx.sparse)
             gx = (gy2 @ (w_eff if w_eff.dtype == gy2.dtype or torch.is_autocast_enabled() else w_eff.to(gy2.dtype)))
             gx = gx.reshape(x.shape).to(x.dtype)
         if ctx.needs_input_grad[2] or ctx.needs_input_grad[3]:
             G = gy2.t() @ x.reshape(-1, x.shape[-1]).to(gy2.dtype)          # dL/dW_eff, in the layer's dtype like autograd
             if G.dtype != W.dtype:
                 G = G.to(W.dtype)
-            dA, dB = native.sparselora_lora_grads(G.contiguous(), Af, Bf, ctx.scaling, mask, ctx.sparse)
+            dA, dB = ctx.source.lora_grads(G.contiguous(), mask, Af, Bf, ctx.scaling, ctx.sparse)
             dA, dB = dA.to(A.dtype), dB.to(B.dtype)
         if ctx.has_bias and ctx.needs_input_grad[4]:
             gbias = gy2.sum(0).to(ctx.bias_dtype)
-        return gx, None, dA, dB, gbias, None, None, None
+        return gx, None, dA, dB, gbias, None, None, None, None
 
 
 class LoraLayer:
@@ -161,7 +176,7 @@ class Linear(nn.Linear, LoraLayer):
                 x = x.to(previous_dtype)
             result = _MaskedLoRALinear.apply(x, self.weight,
                                              self.lora_A.weight, self.lora_B.weight, self.bias, self.mask,
-                                             float(self.scaling), bool(self.sparse))
+                                             float(self.scaling), bool(self.sparse), DenseWeightSource)
         if result.dtype != previous_dtype:
             result = result.to(previous_dtype)
         return result
