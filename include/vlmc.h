@@ -269,7 +269,7 @@ int vlmc_sparselora_lora_grads(const void* G, int dtype, int R, int C, int64_t l
                                float* dA, float* dB, void* ws, size_t ws_bytes, void* stream);
 
 /*
- * Compressed 2:4 weights (K24-K26).  A weight W [R, C] (fp16 / bf16, C % 16 == 0) whose every group of 4 consecutive
+ * Compressed 2:4 weights (K24-K26, K31).  A weight W [R, C] (fp16 / bf16, C % 16 == 0) whose every group of 4 consecutive
  * columns holds at most two non-zeros - what Wanda / SparseGPT / DSnoT leave with prune_n = 2, prune_m = 4 - is stored as
  *   values [R, C/2]   W's dtype.  Group g (columns 4g..4g+3) keeps its two values at [2g, 2g+1], in ascending column order.
  *   meta   [R, C/16]  uint16.  Word j covers columns [16j, 16j+16); group g of the word uses bits [4g, 4g+4): the low
@@ -303,6 +303,25 @@ int vlmc_sparse24_decompress(const void* values, int dtype, int R, int C, int64_
 int vlmc_sparse24_linear_forward(const void* x, int dtype, int64_t T, int C, int64_t ldx, const void* values,
                                  int64_t ldv, const uint16_t* meta, int64_t ldm, int R, const void* bias, void* y,
                                  int64_t ldy, void* ws, size_t ws_bytes, void* stream);
+
+/*
+ * K31  vlmc_sparse24_linear_sp_forward  y[T, R] = x[T, C] . W^T (+ bias[R]) on the sparse tensor cores
+ *      (tcgen05.mma.sp, kind::f16, fp32 accumulation in TMEM), reading values and meta exactly as stored: the weight is
+ *      the sparse operand (M = weight rows), the tokens the dense one.  Each 32-bit TMEM metadata column the instruction
+ *      reads is two consecutive meta words of a row, the lower-column word in the low half - the stored order, no
+ *      reordered copy.  No workspace and no split over K: one CTA owns an output tile and walks K in order, so equal
+ *      inputs give equal bits.  x, values, bias and y share `dtype` (fp16 / bf16); bias may be NULL; y is rounded once,
+ *      after the bias.  C % 32 == 0, R >= 1, any T >= 0; TMA: ldx, ldv, ldm multiples of 8 elements, x / values / meta
+ *      16-byte aligned.  Anything else returns an error and launches nothing.
+ *      Semantics: only the two positions meta names in each group of four take part in the product.  For inputs without
+ *      inf or NaN, y equals x . decompress(values, meta)^T up to fp32 summation order.  An inf or NaN in x at a position
+ *      meta does not name leaves y finite, where the expand path (0 * inf) gives NaN.  Padded positions are named and
+ *      store +0, so there the product is the dense one (0 * inf = NaN).  A meta code whose two indices are both 0 is
+ *      not a 2:4 pattern (the format never writes one); the kernel reads it as indices {0, 1}.
+ */
+int vlmc_sparse24_linear_sp_forward(const void* x, int dtype, int64_t T, int C, int64_t ldx, const void* values,
+                                    int64_t ldv, const uint16_t* meta, int64_t ldm, int R, const void* bias, void* y,
+                                    int64_t ldy, void* stream);
 
 /*
  * SparseLoRA on compressed 2:4 weights (K27-K30).  A SparseLoRA layer pruned with lora_model=True keeps its pruned

@@ -107,11 +107,13 @@ def save_compressed_checkpoint(model, path):
     torch.save({"format": COMPRESSED_FORMAT, "state_dict": state, "sparse24": layers}, path)
 
 
-def load_compressed_checkpoint(model, path, dense=False):
+def load_compressed_checkpoint(model, path, dense=False, sparse_mma=False):
     """Loads a file of save_compressed_checkpoint into `model` (dense or already compressed, same architecture).
     dense=False: the compressed linears become Sparse24Linear (nn.Linears at those names are replaced, on their device).
     dense=True: the weights are expanded (K25, +0 at pruned positions) into the model's nn.Linears, which stay dense, so
-    the result is an ordinary dense state that the reference's loaders take.  Returns the compressed linears' names."""
+    the result is an ordinary dense state that the reference's loaders take.  sparse_mma sets the routing flag of every
+    Sparse24Linear loaded (vlmc.sparse24); the file format does not depend on it.  Returns the compressed linears'
+    names."""
     ckpt = torch.load(path, map_location="cpu")
     if not isinstance(ckpt, dict) or ckpt.get("format") != COMPRESSED_FORMAT:
         raise ValueError(f"{path} is not a {COMPRESSED_FORMAT} checkpoint")
@@ -128,9 +130,11 @@ def load_compressed_checkpoint(model, path, dense=False):
             state[name + ".weight"] = native.sparse24_decompress(values.to(dev), meta.to(dev), C)
             continue
         if isinstance(mod, nn.Linear):
-            new = Sparse24Linear(values.to(dev), meta.to(dev), C, None if bias is None else bias.to(dev))
+            new = Sparse24Linear(values.to(dev), meta.to(dev), C, None if bias is None else bias.to(dev), sparse_mma)
             parent_name, _, child = name.rpartition(".")
             setattr(model.get_submodule(parent_name) if parent_name else model, child, new)
+        else:
+            mod.sparse_mma = bool(sparse_mma)
         state[name + ".values"], state[name + ".meta"] = values, meta
     model.load_state_dict(state)
     return list(layers)

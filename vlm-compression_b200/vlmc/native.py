@@ -65,6 +65,7 @@ SIGNATURES = {
     "vlmc_sparse24_compress": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _vp, _i64, _vp, _vp]),
     "vlmc_sparse24_decompress": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _vp, _i64, _vp]),
     "vlmc_sparse24_linear_forward": (_i, [_vp, _i, _i64, _i, _i64, _vp, _i64, _vp, _i64, _i, _vp, _vp, _i64, _vp, _sz, _vp]),
+    "vlmc_sparse24_linear_sp_forward": (_i, [_vp, _i, _i64, _i, _i64, _vp, _i64, _vp, _i64, _i, _vp, _vp, _i64, _vp]),
     "vlmc_sparse24_compress_masked": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp]),
     "vlmc_sparse24_lora_effective_weight": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _vp, _vp, _i, _f, _i, _vp, _i64, _vp]),
     "vlmc_sparse24_lora_grads": (_i, [_vp, _i, _i, _i, _i64, _vp, _i64, _i, _vp, _vp, _i, _f, _vp, _vp, _vp, _sz, _vp]),
@@ -822,16 +823,9 @@ def sparse24_decompress(values, meta, C, out=None):
     return out
 
 
-def sparse24_linear_supported(x, values, meta, C):
-    """True when K26 takes the call: CUDA tensors, x in the values' fp16 / bf16 dtype, C % 16 == 0, matching shapes."""
-    return (values.is_cuda and meta.is_cuda and x.is_cuda and values.dtype in (torch.float16, torch.bfloat16) and
-            x.dtype == values.dtype and C >= 16 and C % 16 == 0 and x.shape[-1] == C and values.dim() == 2 and
-            values.shape[1] == C // 2 and meta.dtype == torch.int16 and meta.shape == (values.shape[0], C // 16))
-
-
-def sparse24_linear(x, values, meta, C, bias=None, out=None):
-    """K26: y = F.linear(x, decompress(values, meta), bias) read from the compressed weight.  x [..., C] in the values'
-    dtype; returns y [..., R].  Operands whose row pitch TMA cannot take are copied (meta pitch padded to 16 bytes)."""
+def _sparse24_linear_operands(x, values, meta, C, bias, out):
+    """Checks the operands of K26 / K31 and copies those whose row pitch or base TMA cannot take (meta pitch padded to 16
+    bytes).  Returns (R, C, x2 [T, C], values, meta, bias, y [T, R])."""
     R, C = _sparse24_operands(values, meta, C)
     _require_cuda(x)
     if x.dtype != values.dtype or x.shape[-1] != C:
@@ -855,6 +849,21 @@ def sparse24_linear(x, values, meta, C, bias=None, out=None):
     _require_cuda(y)
     if y.dtype != values.dtype or y.shape != (Tn, R) or y.stride(1) != 1:
         raise ValueError("out must be a row-major [T, R] tensor of the values' dtype")
+    return R, C, x2, values, meta, bias, y
+
+
+def sparse24_linear_supported(x, values, meta, C):
+    """True when K26 takes the call: CUDA tensors, x in the values' fp16 / bf16 dtype, C % 16 == 0, matching shapes."""
+    return (values.is_cuda and meta.is_cuda and x.is_cuda and values.dtype in (torch.float16, torch.bfloat16) and
+            x.dtype == values.dtype and C >= 16 and C % 16 == 0 and x.shape[-1] == C and values.dim() == 2 and
+            values.shape[1] == C // 2 and meta.dtype == torch.int16 and meta.shape == (values.shape[0], C // 16))
+
+
+def sparse24_linear(x, values, meta, C, bias=None, out=None):
+    """K26: y = F.linear(x, decompress(values, meta), bias) read from the compressed weight.  x [..., C] in the values'
+    dtype; returns y [..., R].  Operands whose row pitch TMA cannot take are copied (meta pitch padded to 16 bytes)."""
+    R, C, x2, values, meta, bias, y = _sparse24_linear_operands(x, values, meta, C, bias, out)
+    Tn = x2.shape[0]
     if Tn == 0:
         return y.reshape(*x.shape[:-1], R)
     lib = load()
@@ -865,6 +874,31 @@ def sparse24_linear(x, values, meta, C, bias=None, out=None):
                                               bias.data_ptr() if bias is not None else None, y.data_ptr(), y.stride(0),
                                               ws.data_ptr(), ws.numel(), _stream(values))
     _check("vlmc_sparse24_linear_forward", st)
+    return y.reshape(*x.shape[:-1], R)
+
+
+def sparse24_linear_sp_supported(x, values, meta, C):
+    """True when K31 takes the call: sparse24_linear_supported and C % 32 == 0 (whole K = 32 sparse MMAs)."""
+    return sparse24_linear_supported(x, values, meta, C) and C % 32 == 0
+
+
+def sparse24_linear_sp(x, values, meta, C, bias=None, out=None):
+    """K31: y = x . decompress(values, meta)^T (+ bias) on the sparse tensor cores, which multiply only the two positions
+    meta names in each group of four (an inf / NaN of x at an unnamed position does not reach y; include/vlmc.h).  x
+    [..., C] in the values' dtype, C % 32 == 0; returns y [..., R].  Operands whose row pitch TMA cannot take are
+    copied (meta pitch padded to 16 bytes)."""
+    if int(C) % 32:
+        raise ValueError(f"the sparse tensor-core linear needs C % 32 == 0, got C = {C}")
+    R, C, x2, values, meta, bias, y = _sparse24_linear_operands(x, values, meta, C, bias, out)
+    Tn = x2.shape[0]
+    if Tn == 0:
+        return y.reshape(*x.shape[:-1], R)
+    with torch.cuda.device(values.device):
+        st = load().vlmc_sparse24_linear_sp_forward(x2.data_ptr(), _dtype(values), Tn, C, x2.stride(0),
+                                                    values.data_ptr(), values.stride(0), meta.data_ptr(),
+                                                    meta.stride(0), R, bias.data_ptr() if bias is not None else None,
+                                                    y.data_ptr(), y.stride(0), _stream(values))
+    _check("vlmc_sparse24_linear_sp_forward", st)
     return y.reshape(*x.shape[:-1], R)
 
 

@@ -7,6 +7,9 @@ one bit of index per weight (0.5625x the bytes) resident, and multiplies from th
   - from DENSE_EXPAND_MIN_TOKENS tokens on: K25 expands the weight into a scratch buffer shared by all layers on the
     stream, then the library GEMM runs on it.
 Both give y = F.linear(x, W, bias) of the dense pruned weight W within the library GEMM's error; the second bit for bit.
+With sparse_mma=True (opt-in), calls of SPARSE_MMA_MIN_TOKENS <= tokens < SPARSE_MMA_MAX_TOKENS whose in_features is a
+multiple of 32 go to K31 instead, which multiplies values and meta as stored on the sparse tensor cores: no dense scratch buffer, and only
+the positions meta names take part (an inf / NaN of x at a pruned position does not reach y; include/vlmc.h).
 
 SparseLoRA recovery fine-tuning after 2:4 pruning (prune(lora_model=True) -> train the adapters -> merge + re-mask ->
 save) runs on the same format: `Sparse24LoRALinear` holds the frozen weight as values + meta compressed from the layer's
@@ -27,6 +30,12 @@ from vlmc.peft import lora as peft_lora
 # 0.26 against 0.34 ms per block; T = 16: 0.23 against 0.75 ms), so K26 takes no call here until it beats it.
 DENSE_EXPAND_MIN_TOKENS = 1
 
+# Token window in which layers built with sparse_mma=True take K31 (sparse tensor cores) instead of expand + GEMM.
+# Measured on a B200 (1000 W limit), Vicuna-7B block, graph replay (profiles/r05_sparse24_sp_probe.log): K31 beats expand
+# at T = 1 .. 512 (1.44x at T = 1, 1.09x at T = 512) and loses from T = 2048 (0.97x; 0.86x at T = 16384).
+SPARSE_MMA_MIN_TOKENS = 1
+SPARSE_MMA_MAX_TOKENS = 2048
+
 _scratch = {}
 
 
@@ -45,21 +54,22 @@ class Sparse24Linear(nn.Module):
     """Inference-only linear layer on a compressed 2:4 weight: buffers `values` [R, C/2], `meta` [R, C/16] (int16 holding
     the uint16 index words) and optional `bias` [R]."""
 
-    def __init__(self, values, meta, in_features, bias=None):
+    def __init__(self, values, meta, in_features, bias=None, sparse_mma=False):
         super().__init__()
         native._sparse24_operands(values, meta, in_features)
         self.in_features = int(in_features)
         self.out_features = values.shape[0]
+        self.sparse_mma = bool(sparse_mma)          # a routing choice, not state: state_dict() does not hold it
         self.register_buffer("values", values)
         self.register_buffer("meta", meta)
         self.register_buffer("bias", bias)
 
     @classmethod
-    def from_linear(cls, linear):
+    def from_linear(cls, linear, sparse_mma=False):
         """Compresses linear.weight (raises ValueError if it is not 2:4)."""
         values, meta = native.sparse24_compress(linear.weight.detach())
         bias = None if linear.bias is None else linear.bias.detach().to(values.dtype).clone()
-        return cls(values, meta, linear.in_features, bias)
+        return cls(values, meta, linear.in_features, bias, sparse_mma)
 
     def to_dense(self):
         """An nn.Linear holding the expanded weight (+0 at pruned positions)."""
@@ -79,6 +89,9 @@ class Sparse24Linear(nn.Module):
             raise ValueError(f"Sparse24Linear takes [..., {self.in_features}] inputs in {self.values.dtype}, got "
                              f"{list(x.shape)} in {x.dtype}")
         tokens = x.numel() // self.in_features if self.in_features else 0
+        if (self.sparse_mma and SPARSE_MMA_MIN_TOKENS <= tokens < SPARSE_MMA_MAX_TOKENS and
+                native.sparse24_linear_sp_supported(x, self.values, self.meta, self.in_features)):
+            return native.sparse24_linear_sp(x, self.values, self.meta, self.in_features, self.bias)
         if tokens < DENSE_EXPAND_MIN_TOKENS:
             return native.sparse24_linear(x, self.values, self.meta, self.in_features, self.bias)
         W = native.sparse24_decompress(self.values, self.meta, self.in_features,
@@ -86,7 +99,8 @@ class Sparse24Linear(nn.Module):
         return F.linear(x, W, self.bias)
 
     def extra_repr(self):
-        return f"in_features={self.in_features}, out_features={self.out_features}, bias={self.bias is not None}, 2:4"
+        return (f"in_features={self.in_features}, out_features={self.out_features}, bias={self.bias is not None}, 2:4, "
+                f"sparse_mma={self.sparse_mma}")
 
 
 class _Sparse24WeightSource:
@@ -252,12 +266,13 @@ def _lora_swappable(mod):
             1 <= mod.r <= 16 and not mod.merged and not mod.fan_in_fan_out and not mod.disable_adapters)
 
 
-def compress_model(model, lora=False):
+def compress_model(model, lora=False, sparse_mma=False):
     """Replaces, in place, every nn.Linear of `model` whose weight is fp16 / bf16 on a CUDA device, 2:4 sparse and has
     in_features % 16 == 0 by a Sparse24Linear; every other linear stays dense (fp32 ViT linears, unpruned heads, LoRA
     layers).  With lora=True every vlmc.peft.lora.Linear that is fp16 / bf16 on CUDA, has in_features % 16 == 0 and
     1 <= r <= 16, is not merged and whose mask keeps exactly two of every four columns becomes a Sparse24LoRALinear
-    (its lora_A / lora_B go with it and are not listed).  Returns (replaced names, skipped names)."""
+    (its lora_A / lora_B go with it and are not listed).  sparse_mma is passed to every Sparse24Linear (see the module
+    docstring).  Returns (replaced names, skipped names)."""
     replaced, skipped = [], []
     moved = []                                      # prefixes of swapped LoRA layers: their children went with them
     for name, mod in list(model.named_modules()):
@@ -286,7 +301,7 @@ def compress_model(model, lora=False):
             skipped.append(name)
             continue
         try:
-            new = Sparse24Linear.from_linear(mod)
+            new = Sparse24Linear.from_linear(mod, sparse_mma)
         except ValueError:
             skipped.append(name)
             continue
