@@ -483,7 +483,13 @@ int vlmc_chol_set_lookahead(int mode);
  *                                                   else B row-major [K,N]
  *   tri != 0: only tiles touching the lower triangle are computed (symmetric rank-k update of a lower triangle)
  *   kc: K elements accumulated inside the tensor core between round-to-nearest flushes (0 = 128; multiples of 32)
- * K, N, lda, ldb, ldc multiples of 4; pointers 16-byte aligned.
+ *   beta == 0: C is not read (NaN in C does not propagate)
+ * K, N, lda, ldb, ldc multiples of 4; pointers 16-byte aligned; ldc >= N.  Anything else returns an error and launches
+ * nothing.
+ * Non-finite operands: every element a is split into hi = tf32(a) (round to nearest, ties away from zero) and
+ * lo = a - hi.  For a = +-inf, lo = inf - inf is NaN, so every output whose dot product meets an inf or NaN of A or B is
+ * NaN, whatever the other factor (also 0).  Finite values that round past the largest TF32 number (|a| >= 2^128 - 2^116,
+ * e.g. FLT_MAX) split into hi = +-inf and lo = -+inf and behave the same way.  All other outputs are unaffected.
  */
 int vlmc_gemm_tf32x3(int b_nk, int M, int N, int K, float alpha, const float* A, int64_t lda,
                      const float* B, int64_t ldb, float beta, float* C, int64_t ldc, int tri, int kc,

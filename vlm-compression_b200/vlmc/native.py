@@ -1063,16 +1063,25 @@ def gemm_tf32x3(A, B, C=None, alpha=1.0, beta=0.0, b_nk=False, tri=False, kc=0):
     """C = beta * C + alpha * A @ (B.T if b_nk else B) in fp32 on the tensor cores (3xTF32 split, gemm3x.cu).
     A, B, C may be views with a row stride (last dim contiguous)."""
     _require_cuda(A, B, C)
+    if A.dim() != 2 or B.dim() != 2 or (C is not None and C.dim() != 2):
+        raise ValueError("gemm_tf32x3 takes 2-D matrices")
     M, K = A.shape
     N = B.shape[0] if b_nk else B.shape[1]
-    assert (B.shape[1] if b_nk else B.shape[0]) == K
+    if (B.shape[1] if b_nk else B.shape[0]) != K:
+        raise ValueError(f"inner dimensions differ: A is {tuple(A.shape)}, B is {tuple(B.shape)} (b_nk={bool(b_nk)})")
     if C is None:
         C = torch.empty(M, N, device=A.device, dtype=torch.float32)
+    elif C.shape != (M, N):
+        raise ValueError(f"C must be [{M}, {N}], got {tuple(C.shape)}")
     for t in (A, B, C):
-        assert t.dtype == torch.float32 and t.stride(-1) == 1
-    _check("vlmc_gemm_tf32x3", load().vlmc_gemm_tf32x3(
-        int(b_nk), M, N, K, float(alpha), A.data_ptr(), A.stride(0), B.data_ptr(), B.stride(0), float(beta),
-        C.data_ptr(), C.stride(0), int(tri), int(kc), _stream(A)))
+        if t.dtype != torch.float32 or t.stride(-1) != 1:
+            raise ValueError("A, B and C must be float32 matrices with contiguous rows")
+        if t.device != A.device:
+            raise ValueError("A, B and C must be on the same device")
+    with torch.cuda.device(A.device):
+        _check("vlmc_gemm_tf32x3", load().vlmc_gemm_tf32x3(
+            int(b_nk), M, N, K, float(alpha), A.data_ptr(), A.stride(0), B.data_ptr(), B.stride(0), float(beta),
+            C.data_ptr(), C.stride(0), int(tri), int(kc), _stream(A)))
     return C
 
 
