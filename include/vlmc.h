@@ -215,6 +215,9 @@ int vlmc_mask_apply_packed_batch(const vlmc_apply_item* items, int count, int dt
  *   W[r,c] <- keep_mask[r,c] ? round_to_W_dtype( float(W[r,c]) + scaling * sum_k B[r,k]*A[k,c] ) : 0
  * A = lora_A.weight [rank, C], B = lora_B.weight [R, rank], both fp32 row-major contiguous.
  * remask = 0 keeps W[r,c] unchanged where keep_mask is 0 (merge() alone).
+ * The arithmetic: sum_k B A is one fmaf per k, k ascending from +0; then W + (sum * scaling) as two separately rounded
+ * fp32 operations (no contraction), rounded once to W's dtype.  A masked entry is +0 (remask) or W's value as it was,
+ * whatever the LoRA product holds there (see the masked-position rule below K16).
  */
 int vlmc_sparselora_merge(void* W, int dtype, int R, int C, int64_t ldw,
                           const float* A, const float* B, int rank, float scaling,
@@ -223,7 +226,7 @@ int vlmc_sparselora_merge(void* W, int dtype, int R, int C, int64_t ldw,
 
 /*
  * K14 for up to 16 LoRA linears in one launch (train.py:626-637 merges module by module).  `items` is a HOST array
- * read during the call.  rank <= 8; same results as vlmc_sparselora_merge per item.
+ * read during the call.  rank <= 16; same results as vlmc_sparselora_merge per item.
  */
 typedef struct vlmc_merge_item {
   void* W; int64_t ldw; int R; int C;
@@ -237,8 +240,10 @@ int vlmc_sparselora_merge_batch(const vlmc_merge_item* items, int count, int dty
  * (r > 0, not merged), lora.py:364-375, that the reference re-materialises every step:
  *   sparse != 0:  out = ((W + ((B @ A).to(dtype) * scaling)) * mask)        (:364-369)
  *   sparse == 0:  out = ( W * mask + ((B @ A).to(dtype) * scaling))         (:370-375)
- * with the reference's roundings (product cast to W's dtype, scaled in that dtype, added in that dtype).  W is not
- * modified; out [R, C] has W's dtype.  y = F.linear(x, out, bias) stays a library GEMM.
+ * with the reference's roundings (product cast to W's dtype, scaled in that dtype, added in that dtype); the product is
+ * K14's (one fmaf per k, k ascending from +0).  A masked W counts as +0: with sparse != 0 masked entries of out are +0
+ * whatever W or the product hold there (the masked-position rule below K16).  W is not modified; out [R, C] has W's dtype.  y = F.linear(x, out, bias) stays a
+ * library GEMM.
  */
 int vlmc_sparselora_effective_weight(const void* W, int dtype, int R, int C, int64_t ldw, const float* A,
                                      const float* B, int rank, float scaling, const uint8_t* keep_mask,
@@ -262,6 +267,16 @@ int vlmc_sparselora_linear_forward(const void* x, int dtype, int64_t T, int C, i
  * (dy^T x, a library GEMM).  The reference's autograd masks G (sparse only), scales it in W's dtype, casts to fp32 and
  * runs two rank-r GEMMs; here  E = float(round_dtype(G * mask * scaling)),  dB [R, rank] = E A^T,
  * dA [rank, C] = B^T E  in one call (fp32 accumulation, fixed order).  rank <= 16.
+ *
+ * The masked-position rule of K14, K15 and K16, and through them of K23, K28, K29 and K30: a masked W counts as +0,
+ * so masked entries of the sparse effective weight (and of K14's result with remask) are +0 and those of the dense one
+ * are +0 + d; with sparse != 0 a masked entry of G contributes nothing (E = 0 there).  This holds whatever W, the LoRA
+ * product or G hold at that position.  The reference's expressions differ in two ways the values alone do not show:
+ * (W + d) * mask and W * mask give -0 where the masked factor is negative and NaN where it is +-inf, and G * mask turns
+ * an inf or NaN of G into NaN.
+ * K28 and K29 read only the stored kept values, so they cannot know W at a masked position; +0 / nothing is the rule
+ * the whole family can share.  F.linear cannot tell it apart from the reference's, except through 0 * inf in x.
+ * At kept positions inf and NaN propagate as in IEEE arithmetic; NaN payloads are not preserved.
  */
 size_t vlmc_sparselora_lora_grads_workspace_bytes(int R, int C, int rank);
 int vlmc_sparselora_lora_grads(const void* G, int dtype, int R, int C, int64_t ldg, const uint8_t* keep_mask,

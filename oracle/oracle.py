@@ -147,18 +147,34 @@ def wanda_threshold(W32, scaler_row, k_global):
 # ---------------------------------------------------------------------------------------------
 # a8 / K14  SparseLoRA merge + re-mask           lora.py:384-387, train.py:634-637
 # ---------------------------------------------------------------------------------------------
+def _fma32(b, a, c):
+    """fmaf(b, a, c) on float32 arrays, correctly rounded.  The product of two float32 values is exact in float64;
+    TwoSum gives the float64 sum and its exact error, and the sum is rounded to odd (nudged to the odd neighbour when
+    inexact), which makes the final rounding to float32 a single correct one.  float32(float64(b * a) + c) is not: the
+    float64 sum can land exactly on a float32 midpoint (b = 1 - 2^-12 + 2^-24, a = 2^-24 (1 + 2^-12), c = 1 gives 1.0,
+    not 1 + 2^-23)."""
+    p = np.asarray(b, np.float64) * np.asarray(a, np.float64)
+    c = np.asarray(c, np.float64)
+    with np.errstate(invalid="ignore"):
+        s = p + c
+        bb = s - p
+        err = (p - (s - bb)) + (c - bb)
+        even = (s.view(np.int64) & 1) == 0
+        s = np.where(np.isfinite(s) & (err != 0) & even, np.nextafter(s, np.where(err > 0, np.inf, -np.inf)), s)
+    return s.astype(F32)
+
+
 def sparselora_merge(W32, w_tag, A, B, scaling, keep_mask, remask=True):
     """W <- round_w( W + (B@A * scaling) * mask ), then W[~mask] = 0.
 
     fp32 math as torch does it: the rank-r product accumulates k ascending with fused multiply-adds
-    (emulated in float64, exact for one fma, then rounded), `* scaling` and the final add are
-    separately rounded float32 ops, one rounding to W's dtype.
+    (each correctly rounded, _fma32), `* scaling` and the final add are separately rounded float32 ops,
+    one rounding to W's dtype.
     """
     R, C = W32.shape
     acc = np.zeros((R, C), dtype=F32)
     for kk in range(A.shape[0]):
-        prod = B[:, kk].astype(np.float64)[:, None] * A[kk].astype(np.float64)[None, :]
-        acc = (prod + acc.astype(np.float64)).astype(F32)  # fma(b, a, acc) rounded once
+        acc = _fma32(B[:, kk][:, None], A[kk][None, :], acc)
     delta = (acc * F32(scaling)).astype(F32)
     merged = round_to_dtype((W32.astype(F32) + delta).astype(F32), w_tag)
     out = np.where(keep_mask, merged, F32(0) if remask else W32.astype(F32))
@@ -169,11 +185,10 @@ def sparselora_merge(W32, w_tag, A, B, scaling, keep_mask, remask=True):
 # f-2 / K15, K16  SparseLoRA masked training forward and its LoRA gradients      lora.py:359-382
 # ---------------------------------------------------------------------------------------------
 def _lora_product(A, B):
-    """B @ A in float32, k ascending with fused multiply-adds (see sparselora_merge)."""
+    """B @ A in float32, k ascending with one correctly rounded fused multiply-add per step (_fma32)."""
     acc = np.zeros((B.shape[0], A.shape[1]), dtype=F32)
     for kk in range(A.shape[0]):
-        prod = B[:, kk].astype(np.float64)[:, None] * A[kk].astype(np.float64)[None, :]
-        acc = (prod + acc.astype(np.float64)).astype(F32)
+        acc = _fma32(B[:, kk][:, None], A[kk][None, :], acc)
     return acc
 
 
