@@ -517,7 +517,13 @@ int vlmc_gemm_tf32x3(int b_nk, int M, int N, int K, float alpha, const float* A,
  * W (fp16 / bf16 / fp32, [R, C]) is overwritten with the compensated sparse weights (math in fp32, one rounding).
  * dead: optional [C] bytes from vlmc_hessian_prepare (those input channels are zeroed first, :97).
  * keep_mask (optional) receives 1 = kept / 0 = pruned; importance_score (optional) = mean(W^2 / diag(U)^2), :163-165.
- * blocksize must be 128.
+ * Shapes: blocksize must be 128 and C a multiple of 4 (VLMC_ERR_UNSUPPORTED otherwise, as for ldu % 4 != 0 or U not
+ * 16-byte aligned).  The last block may be partial (bs = C mod 128 columns); its threshold rank is int(R * bs * sparsity)
+ * (0-indexed, the double product truncated as Python's int() does) among its R * bs scores.  n:m needs 0 < n < m, m
+ * dividing 128 and m <= 16 (so m is 2, 4, 8 or 16); unstructured needs 0 <= sparsity < 1; both VLMC_ERR_BAD_ARG
+ * otherwise, as is ldm < C.  Arguments are checked before anything is launched.
+ * Every step but the trailing update rounds as the reference's fp32 code: where Err1 @ U[i1:i2, i2:] is exactly zero
+ * (a block-diagonal U, or C <= 128) weights, mask and thresholds equal it bit for bit.  Pruned weights are +0.
  */
 int vlmc_obs_sweep(void* W, int dtype, int R, int C, int64_t ldw, const float* U, int64_t ldu,
                    const uint8_t* dead, double sparsity, int prune_n, int prune_m, int blocksize,
@@ -529,6 +535,8 @@ int vlmc_obs_sweep(void* W, int dtype, int R, int C, int64_t ldw, const float* U
  * device word (vlmc_chol_inv_upper's `status`); when it is non-zero at run time the sweep leaves W and keep_mask
  * untouched (only scratch is written), so the caller can damp, re-factorise and sweep again (sparsegpt_pruner.py:114-128
  * semantics) without a host round trip on the success path.  fail_flag == NULL: identical to vlmc_obs_sweep.
+ * importance_score is computed (by vlmc_obs_begin) before the flag is read, so it is written even when the flag is set:
+ * mean(W^2 / diag(U)^2) of the untouched W and the rejected U.  Nothing the failed call leaves in ws is read by the next.
  */
 int vlmc_obs_sweep_guarded(void* W, int dtype, int R, int C, int64_t ldw, const float* U, int64_t ldu,
                            const uint8_t* dead, double sparsity, int prune_n, int prune_m, int blocksize,

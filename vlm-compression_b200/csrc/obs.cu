@@ -722,6 +722,11 @@ static int obs_block_finish_impl(void* W, int dtype, int R, int C, int64_t ldw, 
       const int behind = C - sb_i2;
       const int next_cols = sb * kOB < behind ? sb * kOB : behind;      // the next super-block's columns
       if (!side || behind - next_cols < kOB) {
+        // the previous super-block's far_rest may still be writing these columns on the side stream
+        if (pending_far && *pending_far) {
+          if (cudaStreamWaitEvent(st, side->updated, 0) != cudaSuccess) return check_launch();
+          *pending_far = false;
+        }
         rc = gemm3x(false, R, behind, K, -1.f, ErrSB, kErrLd, Ufar, ldu, 1.f, l.W32 + sb_i2, C, 0, kc, st);
         if (rc) return rc;
       } else {
